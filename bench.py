@@ -49,6 +49,7 @@ UNIT = "recomputes/s"
 K_PEERS = 5
 B_ALG_APPLY = 76                      # SURVEY 8(d): bytes per applied AppendResponse
 N_ARENAS = 4                          # rotated so consecutive steps never share L2 contents
+DUMP_MAX_GROUPS = 1_500_000           # --dump-outputs writes 32 B per group in all: at most 48 MB
 
 # BASELINE.json configs: groups per GPU, peer slots in the voter union, joint?, seed
 WORKLOADS = {
@@ -163,6 +164,25 @@ def _siblings(cpu: int):
         return {cpu}
 
 
+def dump_outputs(path, n, steps):
+    """steps: {leg: (advanced bitmap u32[], commit index u64[])} of one step.  Writes groups.npy (the group ids, float64:
+    all of them, or a fixed seeded sample of DUMP_MAX_GROUPS), and per leg <leg>_advanced.npy (float32, 1 where the group
+    advanced) and <leg>_commit_index.npy (float64, the group's new commit index; -1 where it did not advance, since the
+    API leaves those entries unspecified)."""
+    os.makedirs(path, exist_ok=True)
+    groups = np.arange(n)
+    if n > DUMP_MAX_GROUPS:
+        groups = np.sort(np.random.default_rng(0).choice(n, DUMP_MAX_GROUPS, replace=False))
+    np.save(os.path.join(path, "groups.npy"), groups.astype(np.float64))
+    for leg, (bm, com) in steps.items():
+        adv = np.unpackbits(bm.view(np.uint8), bitorder="little")[groups].astype(bool)
+        com = com[groups]
+        if np.any(com[adv] >= 1 << 53):
+            raise ValueError(f"{leg}: a commit index is not exact in float64")
+        np.save(os.path.join(path, f"{leg}_advanced.npy"), adv.astype(np.float32))
+        np.save(os.path.join(path, f"{leg}_commit_index.npy"), np.where(adv, com.astype(np.float64), -1.0))
+
+
 def cpu_leg(n_groups, seed, rounds_wanted, threads, budget_s=20.0, joint=False):
     """The oracle (oracle/raft_oracle.c: apply + recompute, range-partitioned over `threads`
     pthreads) on a bounded sample of the same workload.  Only used as the CPU baseline."""
@@ -238,6 +258,10 @@ def main():
     ap.add_argument("--no-sublegs", action="store_true", help="skip recompute_only / scatter / secondary e2e legs")
     ap.add_argument("--profile", action="store_true",
                     help="device-resident loop only (for ncu): no clock warm loop, no e2e, no CPU leg")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step of the fused leg and of `e2e` returned "
+                         "(advanced flag and new commit index per group) as DIR/<name>.npy; DIR/rank<r>/ under several "
+                         "ranks.  Inputs are seeded: the same arguments give the same outputs on every build")
     args = ap.parse_args()
     args.warmup = max(args.warmup, 3)
 
@@ -380,6 +404,13 @@ def main():
         # average duration is the timed region / K (no per-launch event pairs, no Python launch pacing in between)
         ms_total, ms_kernel = timed(step_fused, W, K, per_launch=False)
         n_records = sum(round_len[a][r][1] for a, r in schedule[W:W + K])
+        dumps = {}
+        if args.dump_outputs:    # read now: the scatter and recompute legs reuse the output buffers
+            a = schedule[W + K - 1][0]
+            bm, com = np.empty((n + 31) // 32, dtype=np.uint32), np.empty(n, dtype=np.uint64)
+            arenas[a].d2h(bm, d_outs[a][0])
+            arenas[a].d2h(com, d_outs[a][1])
+            dumps["fused"] = (bm, com)
         sc = ro = None
         if sublegs:
             # scatter: the same streams continue through the general path (no group order needed)
@@ -501,6 +532,8 @@ def main():
         e2e_flags = flags | {"raw": B.STEP_RAW, "packed": B.STEP_ASYNC, "hybrid": B.STEP_ASYNC | B.STEP_HYBRID}[e2e_mode]
         legs["e2e"] = pipelined_leg(lambda j: es.next_round(bufs[j]),
                                     lambda recs: ea.step_begin_records(recs, e2e_flags), chunk)
+        if args.dump_outputs:
+            dumps["e2e"] = tuple(x.copy() for x in ea.step_results(n))
     if e2e_steps and sublegs:
         # e2e_prepacked: the caller already holds the compact stream (pack untimed)
         cap_b = B.compact_bound(rec_slots)
@@ -622,6 +655,8 @@ def main():
                 "sample": f"{done} rounds of the same {args.workload} stream (apply + recompute), {threads} "
                           "pthreads, oracle/raft_oracle.c tuned path (ro_bench_step_fast, == the literal port)"}
         print(json.dumps(line), flush=True)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs if world == 1 else os.path.join(args.dump_outputs, f"rank{rank}"), n, dumps)
     for a in arenas:
         a.close()
     ea.close()
