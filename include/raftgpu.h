@@ -668,8 +668,8 @@ int32_t raftgpu_step_wire_status(raftgpu_arena *arena, const uint8_t **status, u
  * records: pr.update_committed(m.commit), recent_active = true, resume(), a full inflights window of a
  * Replicate peer frees its first entry (INS_FULL clears), and the result byte says whether the reference would
  * call send_append: RAFTGPU_RES_OK | RAFTGPU_RES_SEND when pr.matched < last_index or a snapshot was requested
- * (raft.rs:1800-1803); RAFTGPU_RES_NO_PROGRESS for an unknown peer.  The read-index tail (:1806-1818) is not
- * on this path.  A heartbeat batch is its own pass, ordered by the caller between steps (it reads last_index,
+ * (raft.rs:1800-1803); RAFTGPU_RES_NO_PROGRESS for an unknown peer.  The read-index tail (:1806-1818) is
+ * raftgpu_heartbeat_resp_read (section "ReadIndex" below); this call ignores RAFTGPU_REC_READ_CTX.  A heartbeat batch is its own pass, ordered by the caller between steps (it reads last_index,
  * which a step's LOCAL records write): "all heartbeat responses of the tick after its append responses" is
  * one of the delivery orders raft allows.  One record per (group, peer) cell; a second one is not applied,
  * gets result 0 and -- in the host form -- makes the call return RAFTGPU_ERR_INVALID.
@@ -704,6 +704,121 @@ int32_t raftgpu_arena_enable_inflights(raftgpu_arena *arena, uint32_t max_inflig
 /* One peer's window: *start, *count (inflights.rs:21-23) and, when buffer != NULL, its `capacity` ring entries. */
 int32_t raftgpu_inflights_get(raftgpu_arena *arena, uint32_t group, uint32_t peer_slot, uint32_t *start, uint32_t *count,
                               uint64_t *buffer, uint32_t capacity);
+
+/* ---- ReadIndex (ReadOnlyOption::Safe / LeaseBased, src/read_only.rs) -------- */
+
+/* Keep every group's ReadOnly (read_only.rs:63-68: the queue of pending MsgReadIndex contexts, each with the commit
+ * index it was taken at and its set of heartbeat acknowledgements) in HBM, so that a linearizable read costs no
+ * per-follower host work.  The caller maps each context (m.entries[0].data) to a 64-bit TOKEN -- equal bytes, equal
+ * token within one group's pending set -- and the engine only compares tokens (the same division of labour as the
+ * slot <-> peer-id mapping).  At most `max_pending` (1..64) requests wait per group; the reference has no bound (a
+ * request beyond it is RAFTGPU_READ_FULL and stays with the caller).  Call before groups are allocated.  Memory:
+ * (20 * max_pending + 8) bytes per group, the request pass's scratch word included (168 MB per million groups at 8),
+ * counted in raftgpu_info.device_bytes.  Enabling it routes no step to another kernel.  Every entry point of this section
+ * returns RAFTGPU_ERR_INVALID on an arena without read-index queues.  The passes of one arena run one at a time. */
+int32_t raftgpu_arena_enable_read_index(raftgpu_arena *arena, uint32_t max_pending);
+
+/* One MsgReadIndex as step_leader takes it (raft.rs:2056-2091): 16 bytes.  A peer of a wide group is addressed the
+ * way records address it: (group g + 1, slot s) for peer 8 + s. */
+typedef struct {
+    uint32_t group;
+    uint8_t from_slot; /* slot of m.from (ignored with RAFTGPU_READ_LOCAL) */
+    uint8_t flags;     /* RAFTGPU_READ_LOCAL | RAFTGPU_READ_LEASE */
+    uint16_t reserved;
+    uint64_t ctx;      /* token of m.entries[0].data */
+} raftgpu_read_req;
+/* m.from == INVALID_ID || m.from == self (raft.rs:2791): the answer is a local ReadState, not a MsgReadIndexResp */
+#define RAFTGPU_READ_LOCAL 0x1u
+/* the group runs ReadOnlyOption::LeaseBased (config.rs:117; a per-Raft option the caller knows) */
+#define RAFTGPU_READ_LEASE 0x2u
+
+/* per-request status byte of raftgpu_read_index[_device] */
+#define RAFTGPU_READ_DROPPED 0u         /* !commit_to_current_term (raft.rs:2057-2061), a non-leader included */
+#define RAFTGPU_READ_READY 1u           /* answered now (singleton or LeaseBased, raft.rs:2063-2069 / 2083-2088) */
+#define RAFTGPU_READ_QUEUED 2u          /* ReadOnly::add_request (read_only.rs:86-99): heartbeats carry its ctx */
+#define RAFTGPU_READ_ALREADY_PENDING 3u /* the token is pending already (read_only.rs:88-90): nothing added, the
+                                           caller still broadcasts heartbeats with the ctx (raft.rs:2081) */
+#define RAFTGPU_READ_FULL 4u            /* max_pending requests wait: not queued, the caller keeps the request */
+#define RAFTGPU_READ_SPLIT 5u           /* the group's requests were not contiguous in the batch: this run is not
+                                           applied (resubmit it) */
+#define RAFTGPU_READ_INVALID 6u         /* a group that is not allocated, or from_slot >= 8 on a non-LOCAL request */
+
+/* The MsgReadIndex branch of step_leader for a batch: per request, in batch order within a group, the rules above.
+ * The requests of one group must be contiguous in the batch (a later run of the same group is RAFTGPU_READ_SPLIT);
+ * an INVALID request ends a run.  d_status[i] = RAFTGPU_READ_*; d_index[i] (nullable) = the read index
+ * (raft_log.committed) for READY and QUEUED, 0 otherwise.  Two kernels (scan: the first run of every group;
+ * apply: one thread walks that run), asynchronous on `stream`.  The host form copies, runs and waits; it returns
+ * RAFTGPU_ERR_INVALID when a request came back RAFTGPU_READ_SPLIT (every other request was applied). */
+int32_t raftgpu_read_index_device(raftgpu_arena *arena, void *stream, const raftgpu_read_req *d_reqs, uint64_t n,
+                                  uint8_t *d_status, uint64_t *d_index);
+int32_t raftgpu_read_index(raftgpu_arena *arena, const raftgpu_read_req *reqs, uint64_t n, uint8_t *status,
+                           uint64_t *index);
+
+/* A flag on RAFTGPU_REC_HEARTBEAT records: the MsgHeartbeatResponse carries a non-empty context (raft.rs:1805), and
+ * `index` carries its token.  Without it the read tail is skipped.  raftgpu_heartbeat_resp[_device] ignores it. */
+#define RAFTGPU_REC_READ_CTX 0x08u
+
+/* ReadOnly::recv_ack (read_only.rs:104-109) for a batch of heartbeat responses: every HEARTBEAT | READ_CTX record
+ * whose peer has a Progress (raft.rs:1779-1789) adds its peer to the ack set of the pending request with that token
+ * (an unknown token is ignored) and marks the request "acknowledged in this batch".  Acks form a set: a duplicate
+ * record changes nothing.  One thread per record, asynchronous on `stream`. */
+int32_t raftgpu_read_ack_device(raftgpu_arena *arena, void *stream, const raftgpu_append_resp *d_records, uint64_t n);
+
+/* One released request: a ReadState (RAFTGPU_READ_LOCAL) or a MsgReadIndexResp to `to_slot` (raft.rs:2790-2806).
+ * 24 bytes; to_slot of a wide group's peer 8 + s is s on group g + 1, like records. */
+typedef struct {
+    uint32_t group;
+    uint8_t to_slot;
+    uint8_t flags;     /* RAFTGPU_READ_LOCAL */
+    uint16_t reserved;
+    uint64_t index;    /* ReadIndexStatus::index: the commit index when the request was queued */
+    uint64_t ctx;      /* the request's token */
+} raftgpu_read_state;
+
+/* ReadOnly::advance (read_only.rs:114-129) behind ProgressTracker::has_quorum (tracker.rs:367-372) for groups
+ * [first, first + n): per group, the requests up to and including the LAST one that was acknowledged since the
+ * previous release pass and whose ack set is a quorum of the current (joint) configuration are released -- for a
+ * batch of heartbeat responses the same requests the reference releases one response at a time.  A request that
+ * was not acknowledged in the batch is not released even if its set is a quorum (the reference checks only the
+ * acked context).  The pass clears the "acknowledged" marks.  Released requests go to d_out as a stream compaction:
+ * the states of one group are contiguous and in queue order, groups in no particular order.  d_count[0] = states
+ * the pass released or wanted to, d_count[1] = states written (a prefix of d_out); d_count[0] > capacity means
+ * that the groups that did not fit kept their queues and marks: call again.  Asynchronous on `stream`.
+ * The host form runs over all allocated groups: *out_n = states written to `out`; RAFTGPU_ERR_FULL when groups
+ * did not fit (they are released by the next call). */
+int32_t raftgpu_read_release_device(raftgpu_arena *arena, void *stream, uint32_t first, uint32_t n,
+                                    raftgpu_read_state *d_out, uint64_t capacity, uint64_t *d_count);
+int32_t raftgpu_read_release(raftgpu_arena *arena, raftgpu_read_state *out, uint64_t capacity, uint64_t *out_n);
+
+/* The whole of Raft::handle_heartbeat_response (raft.rs:1777-1818) for a batch: raftgpu_heartbeat_resp's tracker
+ * part (result bytes into `results`, nullable), then recv_ack, then the release pass over all allocated groups
+ * (states as raftgpu_read_release).  Returns RAFTGPU_ERR_FULL as raftgpu_read_release, else RAFTGPU_ERR_INVALID
+ * when a (group, peer) cell had two records (as raftgpu_heartbeat_resp; the ack of the second is a no-op). */
+int32_t raftgpu_heartbeat_resp_read(raftgpu_arena *arena, const raftgpu_append_resp *records, uint64_t n,
+                                    uint8_t *results, raftgpu_read_state *states, uint64_t capacity,
+                                    uint64_t *out_n);
+
+/* ReadOnly::last_pending_request_ctx (read_only.rs:132-134) for groups [first, first + n): the context
+ * bcast_heartbeat attaches (raft.rs:876).  d_out[g - first] = token, RAFTGPU_NO_READ_CTX when the queue is empty
+ * (so token 0 can stand for the empty context).  Asynchronous on `stream`. */
+#define RAFTGPU_NO_READ_CTX UINT64_MAX
+int32_t raftgpu_read_index_last_ctx_device(raftgpu_arena *arena, void *stream, uint32_t first, uint32_t n,
+                                           uint64_t *d_out);
+
+/* The read tail of Raft::post_conf_change (raft.rs:2648-2664), where the reference reaches raft.rs:2650 (after
+ * raftgpu_group_set_conf): the self peer acks the LAST pending request, and when its ack set is a quorum of the new
+ * configuration every pending request is released into `out`.  Synchronous, one group.  RAFTGPU_ERR_FULL (nothing
+ * released, *out_n = the number needed) when `capacity` is too small. */
+int32_t raftgpu_group_read_index_conf_changed(raftgpu_arena *arena, uint32_t group, raftgpu_read_state *out,
+                                              uint64_t capacity, uint64_t *out_n);
+
+/* One group's queue in order, for tests and inspection: *out_n pending requests; when the arrays are non-NULL
+ * (room for `capacity`), ctx[k], index[k] and word[k] of the k-th one, word = ack mask over peer slots 0..15 in bits
+ * 0..15 | from slot << 16 | RAFTGPU_READ_WORD_* flags. */
+#define RAFTGPU_READ_WORD_LOCAL 0x01000000u /* RAFTGPU_READ_LOCAL request */
+#define RAFTGPU_READ_WORD_ACKED 0x02000000u /* acknowledged since the last release pass */
+int32_t raftgpu_read_index_get(raftgpu_arena *arena, uint32_t group, uint64_t *ctx, uint64_t *index, uint32_t *word,
+                               uint32_t capacity, uint32_t *out_n);
 
 /* ---- votes (SURVEY 8(f) rank 1) ----------------------------------------- */
 

@@ -54,6 +54,16 @@ SEND_ENTRY_DTYPE = np.dtype([("group", "<u4"), ("peer_slot", "u1"), ("flags", "u
                              ("next_idx", "<u8")])
 assert SEND_ENTRY_DTYPE.itemsize == 16
 SEND_SNAPSHOT = 0x1
+READ_REQ_DTYPE = np.dtype([("group", "<u4"), ("from_slot", "u1"), ("flags", "u1"), ("reserved", "<u2"), ("ctx", "<u8")])
+assert READ_REQ_DTYPE.itemsize == 16
+READ_STATE_DTYPE = np.dtype([("group", "<u4"), ("to_slot", "u1"), ("flags", "u1"), ("reserved", "<u2"),
+                             ("index", "<u8"), ("ctx", "<u8")])
+assert READ_STATE_DTYPE.itemsize == 24
+READ_LOCAL, READ_LEASE = 0x1, 0x2
+READ_DROPPED, READ_READY, READ_QUEUED, READ_ALREADY_PENDING, READ_FULL, READ_SPLIT, READ_INVALID = range(7)
+REC_READ_CTX = 0x08
+READ_WORD_LOCAL, READ_WORD_ACKED = 0x01000000, 0x02000000
+NO_READ_CTX = U64_MAX
 
 # host column name -> (column id, numpy dtype, per-peer?)
 COLUMNS = {
@@ -277,6 +287,16 @@ def lib() -> C.CDLL:
             "raftgpu_wire_apply_device": ([vp, vp, vp, u64, vp, u64, vp], i32),
             "raftgpu_step_begin_wire": ([vp, C.POINTER(WireBatch), u32], i32),
             "raftgpu_step_wire_status": ([vp, C.POINTER(vp), C.POINTER(u64)], i32),
+            "raftgpu_arena_enable_read_index": ([vp, u32], i32),
+            "raftgpu_read_index_device": ([vp, vp, vp, u64, vp, vp], i32),
+            "raftgpu_read_index": ([vp, vp, u64, vp, vp], i32),
+            "raftgpu_read_ack_device": ([vp, vp, vp, u64], i32),
+            "raftgpu_read_release_device": ([vp, vp, u32, u32, vp, u64, vp], i32),
+            "raftgpu_read_release": ([vp, vp, u64, C.POINTER(u64)], i32),
+            "raftgpu_heartbeat_resp_read": ([vp, vp, u64, vp, vp, u64, C.POINTER(u64)], i32),
+            "raftgpu_read_index_last_ctx_device": ([vp, vp, u32, u32, vp], i32),
+            "raftgpu_group_read_index_conf_changed": ([vp, u32, vp, u64, C.POINTER(u64)], i32),
+            "raftgpu_read_index_get": ([vp, u32, vp, vp, vp, u32, C.POINTER(u32)], i32),
             "raftgpu_counters_read": ([vp, C.POINTER(Counters)], i32),
             "raftgpu_synchronize": ([vp], i32),
             "raftgpu_debug_read": ([vp, vp], i32),
@@ -772,6 +792,67 @@ class Arena:
             self._ck(self._L.raftgpu_step_record_results(self._h, ring, out.ctypes.data, n.value,
                                                          C.byref(n)), "step_record_results")
         return out
+
+    # -- ReadIndex (ReadOnly queues in HBM)
+    def enable_read_index(self, max_pending: int):
+        self._ck(self._L.raftgpu_arena_enable_read_index(self._h, max_pending), "arena_enable_read_index")
+        self.rd_cap = max_pending
+
+    def read_index(self, reqs: np.ndarray, check: bool = True):
+        """raftgpu_read_index: requests -> (status bytes, read indexes).  check=False returns a SPLIT batch's results
+        instead of raising."""
+        assert reqs.dtype == READ_REQ_DTYPE and reqs.flags.c_contiguous
+        st, idx = np.zeros(len(reqs), dtype=np.uint8), np.zeros(len(reqs), dtype=np.uint64)
+        rc = self._L.raftgpu_read_index(self._h, reqs.ctypes.data, len(reqs), st.ctypes.data, idx.ctypes.data)
+        if check or rc != ERR_INVALID:
+            self._ck(rc, "read_index")
+        return st, idx
+
+    def read_release(self, capacity: int):
+        """raftgpu_read_release -> (states, complete: False when groups did not fit and wait for the next call)."""
+        out, n = np.zeros(capacity, dtype=READ_STATE_DTYPE), C.c_uint64()
+        rc = self._L.raftgpu_read_release(self._h, out.ctypes.data if capacity else None, capacity, C.byref(n))
+        if rc != ERR_FULL:
+            self._ck(rc, "read_release")
+        return out[: n.value], rc == OK
+
+    def heartbeat_resp_read(self, recs: np.ndarray, capacity: int):
+        """raftgpu_heartbeat_resp_read -> (result bytes, released states, complete)."""
+        assert recs.dtype == APPEND_RESP_DTYPE and recs.flags.c_contiguous
+        res, out, n = np.zeros(len(recs), dtype=np.uint8), np.zeros(capacity, dtype=READ_STATE_DTYPE), C.c_uint64()
+        rc = self._L.raftgpu_heartbeat_resp_read(self._h, recs.ctypes.data, len(recs), res.ctypes.data,
+                                                 out.ctypes.data if capacity else None, capacity, C.byref(n))
+        if rc != ERR_FULL:
+            self._ck(rc, "heartbeat_resp_read")
+        return res, out[: n.value], rc == OK
+
+    def read_index_device(self, d_reqs, n, d_status, d_index=None, stream=None):
+        self._ck(self._L.raftgpu_read_index_device(self._h, stream, d_reqs, n, d_status, d_index), "read_index_device")
+
+    def read_ack_device(self, d_records, n, stream=None):
+        self._ck(self._L.raftgpu_read_ack_device(self._h, stream, d_records, n), "read_ack_device")
+
+    def read_release_device(self, first, n, d_out, capacity, d_count, stream=None):
+        self._ck(self._L.raftgpu_read_release_device(self._h, stream, first, n, d_out, capacity, d_count),
+                 "read_release_device")
+
+    def read_index_last_ctx_device(self, first, n, d_out, stream=None):
+        self._ck(self._L.raftgpu_read_index_last_ctx_device(self._h, stream, first, n, d_out), "read_index_last_ctx_device")
+
+    def read_index_conf_changed(self, g, capacity: int = 64) -> np.ndarray:
+        out, n = np.zeros(capacity, dtype=READ_STATE_DTYPE), C.c_uint64()
+        self._ck(self._L.raftgpu_group_read_index_conf_changed(self._h, g, out.ctypes.data, capacity, C.byref(n)),
+                 "group_read_index_conf_changed")
+        return out[: n.value]
+
+    def read_index_get(self, g):
+        """One group's pending requests in queue order: (ctx u64[], index u64[], word u32[])."""
+        cap = self.rd_cap
+        ctx, idx, word, n = (np.zeros(cap, dtype=np.uint64), np.zeros(cap, dtype=np.uint64),
+                             np.zeros(cap, dtype=np.uint32), C.c_uint32())
+        self._ck(self._L.raftgpu_read_index_get(self._h, g, ctx.ctypes.data, idx.ctypes.data, word.ctypes.data, cap,
+                                                C.byref(n)), "read_index_get")
+        return ctx[: n.value], idx[: n.value], word[: n.value]
 
     # -- votes
     def reset_votes(self, g):

@@ -558,6 +558,11 @@ void destroy(raftgpu_arena *a) {
     cudaFree(c.term);
     cudaFree(c.ins_meta);
     cudaFree(c.ins_buf);
+    cudaFree(c.rd_meta);
+    cudaFree(c.rd_ctx);
+    cudaFree(c.rd_index);
+    cudaFree(c.rd_word);
+    cudaFree(c.rd_first);
     cudaFree(a->d_wire_first);
     cudaFree(a->d_counters);
     cudaFree(a->d_scratch);
@@ -753,6 +758,15 @@ int32_t sync_op(raftgpu_arena *a, F &&launch) {
     return RAFTGPU_OK;
 }
 
+// Group alloc / free on an arena with read-index queues: the groups' queues are empty and marked (un)allocated.
+int32_t read_mark_alloc(raftgpu_arena *a, uint32_t first, uint32_t n, bool allocated) {
+    if (!a->cols.rd_cap || n == 0) return RAFTGPU_OK;
+    const uint32_t blocks = std::min<uint32_t>(div_up(n, 256), 8u * static_cast<uint32_t>(a->sm_count));
+    return sync_op(a, [&](cudaStream_t st) {
+        read_alloc_kernel<<<blocks, 256, 0, st>>>(a->cols, first, n, allocated ? kRdAlloc : 0u);
+    });
+}
+
 struct ColumnDesc {
     void *base;
     size_t elem;
@@ -856,5 +870,6 @@ extern "C" {
 #include "abi_compact.inc"
 #include "abi_wire.inc"
 #include "abi_results.inc"
+#include "abi_read.inc"
 
 }  // extern "C"

@@ -25,6 +25,15 @@ struct Columns {
     uint32_t ins_cap;
     uint32_t *ins_meta;
     uint64_t *ins_buf;
+    // ReadOnly queues (raftgpu_arena_enable_read_index; k_read.cuh): rd_cap = max_pending, 0 = off; rd_meta [cap] =
+    // head | count << 16 | kRdAlloc; rd_ctx / rd_index / rd_word [rd_cap][cap] by ring position; rd_first [cap] the
+    // request pass's scratch (UINT32_MAX between passes)
+    uint32_t rd_cap;
+    uint32_t *rd_meta;
+    uint64_t *rd_ctx;
+    uint64_t *rd_index;
+    uint32_t *rd_word;
+    uint32_t *rd_first;
 };
 
 enum Counter : int {
@@ -88,6 +97,29 @@ __device__ __forceinline__ bool ins_add(const Columns &c, size_t cell, uint64_t 
     c.ins_meta[cell] = start | ((count + 1) << 16);
     if (count + 1 == c.ins_cap) flags |= RAFTGPU_PF_INS_FULL;
     return true;
+}
+
+// ---------------------------------------------------------------------------
+// ReadOnly queues (k_read.cuh): the layout constants and the two control-plane hooks, no-ops on arenas without queues.
+constexpr uint32_t kRdAlloc = 0x80000000u;  // rd_meta: the group slot is allocated (a request for any other is INVALID)
+constexpr uint32_t kRdAckMask = 0xffffu;    // rd_word: acks over peer slots 0..15
+constexpr uint32_t kRdFromShift = 16;       // rd_word: from slot (0..15) in bits 16..23
+__device__ __forceinline__ uint32_t rd_head(uint32_t m) { return m & 0xffu; }
+__device__ __forceinline__ uint32_t rd_count(uint32_t m) { return (m >> 16) & 0xffu; }
+// apply_conf removed peer slots `removed` of the half `g` whose new meta word is `meta`: their acks leave every pending
+// request of the group (the queue lives on the low half of a wide group, where peer 8 + s is ack bit 8 + s)
+__device__ __forceinline__ void rd_clear_slots(const Columns &c, uint32_t g, uint32_t meta, uint32_t removed) {
+    if (!c.rd_cap || !removed) return;
+    const bool hi = (meta & RAFTGPU_META_WIDE_HI) != 0;
+    const uint32_t lo = hi ? g - 1 : g, clear = removed << (hi ? 8 : 0);
+    for (uint32_t p = 0; p < c.rd_cap; p++) {
+        uint32_t *w = &c.rd_word[static_cast<size_t>(p) * c.cap + lo];
+        if (*w & clear) *w &= ~clear;
+    }
+}
+// Raft::reset replaces the ReadOnly (raft.rs:957)
+__device__ __forceinline__ void rd_empty(const Columns &c, uint32_t g) {
+    if (c.rd_cap) c.rd_meta[g] &= kRdAlloc;
 }
 
 // ---------------------------------------------------------------------------

@@ -272,6 +272,7 @@ __global__ void conf_kernel(Columns c, uint32_t g, uint32_t new_meta, uint32_t a
             ins_reset(c, cell);  // Inflights::new(max_inflight), progress.rs:70
         }
     }
+    rd_clear_slots(c, g, new_meta, removed);  // acks are by peer id: a later occupant of the slot must not inherit them
     c.meta[g] = new_meta;
 }
 
@@ -296,6 +297,7 @@ __global__ void reset_kernel(Columns c, uint32_t g, uint64_t term_start, uint64_
             c.peer_committed[cell] = committed;  // raft.rs:968
         }
     }
+    rd_empty(c, g);  // raft.rs:957 read_only = ReadOnly::new(..)
     c.committed[g] = committed;
     c.term_start[g] = term_start;
     c.last_index[g] = last_index;

@@ -22,5 +22,6 @@ namespace raftgpu {
 #include "k_tile_compact.cuh"
 #include "k_control.cuh"
 #include "k_wire.cuh"
+#include "k_read.cuh"
 
 }  // namespace raftgpu
