@@ -384,10 +384,8 @@ int32_t raftgpu_apply_device_packed(raftgpu_arena *arena, void *stream, const vo
  * (raftgpu_tile_index builds and validates it on the host).  One wave per call, like
  * raftgpu_apply_device; processes all allocated groups [0, hi).  A record found outside its tile
  * is not applied and reported as RAFTGPU_RES_NO_PROGRESS.  Asynchronous on `stream`. */
-#ifndef RAFTGPU_TILE_GROUPS
 #define RAFTGPU_TILE_GROUPS 256
-#endif
-uint32_t raftgpu_tile_groups(void); /* the value the library was built with */
+uint32_t raftgpu_tile_groups(void); /* RAFTGPU_TILE_GROUPS, as the library sees it */
 int32_t raftgpu_step_sorted_device(raftgpu_arena *arena, void *stream, const void *d_packed_records,
                                    uint64_t n_packed, const uint32_t *d_tile_off, uint8_t *d_results,
                                    uint32_t *d_adv_bitmap, uint64_t *d_commit_out);

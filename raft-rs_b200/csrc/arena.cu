@@ -227,12 +227,7 @@ struct raftgpu_arena {
     bool rec_fallback_sorted = false;        // raftgpu_step_begin_records: the batch going to the general staging path is in group order
     uint32_t n_wide = 0;                     // wide groups (two slots each): the fused tile kernels are not used while any exist
     uint32_t n_simple5 = 0;                  // groups whose meta is the plain 5-voter configuration
-    bool force_general = false;              // RAFTGPU_FORCE_GENERAL=1: never take the simple5 kernels
-    bool prefetch = false;                   // RAFTGPU_PREFETCH=1: kernels with the L2 prefetch stage
-    bool use_tma = false;                    // RAFTGPU_TMA=1 selects the TMA-fed recompute kernel
-    uint32_t tma_smem = 0;                   // dynamic shared memory for the TMA stage ring
-    uint32_t tile_smem = 0;                  // dynamic shared memory for the fused tile kernel
-    int tma_stages_cap = 0;                  // RAFTGPU_TMA_STAGES (tuning knob)
+    uint32_t tile_smem = 0;                  // dynamic shared memory for the fused tile kernels
     Columns cols{};
     uint32_t *d_wire_first = nullptr;  // [kSlots][cap] wire steps: first frame of every cell (allocated on first use)
     unsigned long long *d_counters = nullptr;
@@ -414,22 +409,16 @@ inline bool resolve_slot(const raftgpu_arena *a, uint32_t g, uint32_t slot, uint
 inline bool range_simple5(const raftgpu_arena *a, uint32_t first, uint32_t n) {
     return a->n_simple5 == a->hi && static_cast<uint64_t>(first) + n <= a->hi;
 }
-// Tuning / diagnostic knobs of the fused tile kernel, read once per process -- or on every launch when
-// RAFTGPU_TILE_TUNE is set (scripts/micro_tile.py sweeps them inside one process).
-//   RAFTGPU_TILE_VARIANT = <threads per consumer group><groups> (2563 = 256 x 3), _RECCAP = records staged per tile
-//   (0: read directly), _STAGES, _DEBUG (phase cycle counters), _SKIP (diagnostics, wrong results)
+// Diagnostic knobs of the fused tile kernels, read once per process -- or on every launch when
+// RAFTGPU_TILE_TUNE is set (scripts/micro_tile.py switches them inside one process).
+//   RAFTGPU_TILE_DEBUG (phase cycle counters), _SKIP (phases left out: results are WRONG)
 struct TileKnobs {
-    int variant, cap, stages;
     bool debug;
     uint32_t skip;
 };
 inline TileKnobs read_tile_knobs() {
-    auto num = [](const char *name, int dflt) {
-        const char *v = getenv(name);
-        return v ? atoi(v) : dflt;
-    };
-    return TileKnobs{num("RAFTGPU_TILE_VARIANT", 2563), num("RAFTGPU_TILE_RECCAP", 0), num("RAFTGPU_TILE_STAGES", kFMaxStages),
-                     getenv("RAFTGPU_TILE_DEBUG") != nullptr, static_cast<uint32_t>(num("RAFTGPU_TILE_SKIP", 0))};
+    const char *skip = getenv("RAFTGPU_TILE_SKIP");
+    return TileKnobs{getenv("RAFTGPU_TILE_DEBUG") != nullptr, static_cast<uint32_t>(skip ? atoi(skip) : 0)};
 }
 inline const TileKnobs &tile_knobs() {
     static const bool tune = getenv("RAFTGPU_TILE_TUNE") != nullptr;
@@ -449,36 +438,11 @@ int32_t launch_recompute(raftgpu_arena *a, cudaStream_t st, uint32_t first, uint
                          uint32_t *d_adv, uint64_t *d_commit, uint64_t *d_mci, uint8_t *d_gc,
                          uint32_t *d_step_adv) {
     if (n == 0) return RAFTGPU_OK;
-    const bool simple5 = range_simple5(a, first, n) && !a->force_general;
+    const bool simple5 = range_simple5(a, first, n);
     if (simple5) hint = 0x1fu;
-    if (a->use_tma && a->n_wide == 0 && n >= 16u * kTile && hint != 0) {
-        // TMA-fed pipeline: one persistent CTA per SM, as many stages as fit in shared memory
-        const uint32_t stage_bytes =
-            (static_cast<uint32_t>(__builtin_popcount(hint & 0xffu)) + 3u) * kTile * 8u + kTile * 4u;
-        int stages = std::min<int>(kMaxStages, static_cast<int>(a->tma_smem / stage_bytes));
-        if (a->tma_stages_cap > 0) stages = std::min(stages, a->tma_stages_cap);
-        if (stages >= 2) {
-            const uint32_t base = first - (first % kTile);
-            const uint32_t tiles = div_up(static_cast<uint64_t>(first - base) + n, kTile);
-            const uint32_t blocks = std::min<uint32_t>(tiles, static_cast<uint32_t>(a->sm_count));
-            const size_t smem = static_cast<size_t>(stages) * stage_bytes;
-            if (simple5)
-                recompute_tma_kernel<true><<<blocks, kTmaThreads, smem, st>>>(
-                    a->cols, first, n, hint, stages, d_adv, d_commit, d_mci, d_gc, d_step_adv, a->d_counters);
-            else
-                recompute_tma_kernel<false><<<blocks, kTmaThreads, smem, st>>>(
-                    a->cols, first, n, hint, stages, d_adv, d_commit, d_mci, d_gc, d_step_adv, a->d_counters);
-            CKL(a);
-            return RAFTGPU_OK;
-        }
-    }
     const uint32_t base = first & ~31u;
     const uint64_t threads = static_cast<uint64_t>(first - base) + n;
-    if (simple5 && a->prefetch) {
-        const uint32_t blocks = std::min<uint32_t>(div_up(threads, 256), static_cast<uint32_t>(a->grid_recompute5));
-        recompute_kernel<true, true><<<blocks, 256, 0, st>>>(a->cols, first, n, hint, d_adv, d_commit, d_mci, d_gc,
-                                                            d_step_adv, a->d_counters);
-    } else if (simple5) {
+    if (simple5) {
         const uint32_t blocks = std::min<uint32_t>(div_up(threads, 256), static_cast<uint32_t>(a->grid_recompute5));
         recompute_kernel<true><<<blocks, 256, 0, st>>>(a->cols, first, n, hint, d_adv, d_commit, d_mci, d_gc,
                                                       d_step_adv, a->d_counters);
@@ -495,12 +459,8 @@ int32_t launch_apply(raftgpu_arena *a, cudaStream_t st, const void *d_recs, uint
                      bool packed) {
     if (n == 0) return RAFTGPU_OK;
     const uint32_t blocks = std::min<uint32_t>(div_up(n, 256), static_cast<uint32_t>(a->grid_apply));
-    if (packed && a->prefetch)
-        apply_kernel<true, false, true><<<blocks, 256, 0, st>>>(a->cols, d_recs, n, d_results, a->d_counters);
-    else if (packed)
+    if (packed)
         apply_kernel<true><<<blocks, 256, 0, st>>>(a->cols, d_recs, n, d_results, a->d_counters);
-    else if (a->prefetch)
-        apply_kernel<false, false, true><<<blocks, 256, 0, st>>>(a->cols, d_recs, n, d_results, a->d_counters);
     else
         apply_kernel<false><<<blocks, 256, 0, st>>>(a->cols, d_recs, n, d_results, a->d_counters);
     CKL(a);
@@ -632,57 +592,17 @@ int32_t create(int32_t device, uint32_t max_groups, uint32_t slots, uint32_t n_r
     a->grid_recompute5 = std::max(1, occ) * a->sm_count;
     TRYC(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, apply_kernel<true>, 256, 0));
     a->grid_apply = std::max(1, occ) * a->sm_count;
-    a->tma_smem = 200u * 1024u;
-    TRYC(cudaFuncSetAttribute(recompute_tma_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                              static_cast<int>(a->tma_smem)));
-    TRYC(cudaFuncSetAttribute(recompute_tma_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                              static_cast<int>(a->tma_smem)));
     a->tile_smem = 227u * 1024u - 5u * 1024u;  // 227 KB per CTA minus the kernels' static shared memory (barriers, deferred lists)
-#define RAFTGPU_TILE_ATTR(CT, NG)                                                                             \
-    TRYC(cudaFuncSetAttribute(step_tile_kernel<false, CT, NG>, cudaFuncAttributeMaxDynamicSharedMemorySize,  \
-                              static_cast<int>(a->tile_smem)));                                              \
-    TRYC(cudaFuncSetAttribute(step_tile_kernel<true, CT, NG>, cudaFuncAttributeMaxDynamicSharedMemorySize,   \
-                              static_cast<int>(a->tile_smem)))
-#if RAFTGPU_TILE_GROUPS == 192
-    RAFTGPU_TILE_ATTR(192, 3);
-    RAFTGPU_TILE_ATTR(192, 4);
-    RAFTGPU_TILE_ATTR(192, 5);
-#elif RAFTGPU_TILE_GROUPS == 128
-    RAFTGPU_TILE_ATTR(128, 3);
-    RAFTGPU_TILE_ATTR(128, 4);
-    RAFTGPU_TILE_ATTR(128, 6);
-    RAFTGPU_TILE_ATTR(256, 2);
-    RAFTGPU_TILE_ATTR(256, 3);
-#else
-    RAFTGPU_TILE_ATTR(256, 1);
-    RAFTGPU_TILE_ATTR(256, 2);
-    RAFTGPU_TILE_ATTR(256, 3);
-    RAFTGPU_TILE_ATTR(512, 1);
-#endif
-#undef RAFTGPU_TILE_ATTR
-#define RAFTGPU_CTILE_ATTR(NG)                                                                                   \
-    TRYC(cudaFuncSetAttribute(step_tile_compact_kernel<false, NG, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, \
-                              static_cast<int>(a->tile_smem)));                                                      \
-    TRYC(cudaFuncSetAttribute(step_tile_compact_kernel<true, NG, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,  \
-                              static_cast<int>(a->tile_smem)));                                                      \
-    TRYC(cudaFuncSetAttribute(step_tile_compact_kernel<false, NG, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,  \
-                              static_cast<int>(a->tile_smem)));                                                      \
-    TRYC(cudaFuncSetAttribute(step_tile_compact_kernel<true, NG, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,   \
-                              static_cast<int>(a->tile_smem)))
-    RAFTGPU_CTILE_ATTR(1);
-    RAFTGPU_CTILE_ATTR(2);
-    RAFTGPU_CTILE_ATTR(3);
-#undef RAFTGPU_CTILE_ATTR
-    {
-        const char *e = getenv("RAFTGPU_TMA");
-        a->use_tma = e && e[0] == '1';
-        const char *f = getenv("RAFTGPU_FORCE_GENERAL");
-        a->force_general = f && f[0] == '1';
-        const char *pf = getenv("RAFTGPU_PREFETCH");
-        a->prefetch = pf && pf[0] == '1';
-        const char *t = getenv("RAFTGPU_TMA_STAGES");
-        if (t) a->tma_stages_cap = atoi(t);
-    }
+    TRYC(cudaFuncSetAttribute(step_tile_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(a->tile_smem)));
+    TRYC(cudaFuncSetAttribute(step_tile_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(a->tile_smem)));
+    TRYC(cudaFuncSetAttribute(step_tile_compact_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                              static_cast<int>(a->tile_smem)));
+    TRYC(cudaFuncSetAttribute(step_tile_compact_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                              static_cast<int>(a->tile_smem)));
+    TRYC(cudaFuncSetAttribute(step_tile_compact_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                              static_cast<int>(a->tile_smem)));
+    TRYC(cudaFuncSetAttribute(step_tile_compact_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                              static_cast<int>(a->tile_smem)));
     TRYC(cudaStreamCreateWithFlags(&a->s_compute, cudaStreamNonBlocking));
     TRYC(cudaStreamCreateWithFlags(&a->s_h2d, cudaStreamNonBlocking));
     TRYC(cudaStreamCreateWithFlags(&a->s_d2h, cudaStreamNonBlocking));

@@ -30,7 +30,7 @@ __device__ __forceinline__ void reset_state(const Columns &c, size_t cell, Cell 
 //                        the cell loads (meta, matched, next_idx, pflags,
 //                        committed_index) of element k+1,
 //   and computes / stores element k,
-// so every load has a whole iteration to land.  (An extra L2-prefetch stage, kPrefetch, was
+// so every load has a whole iteration to land.  (An extra L2-prefetch stage was
 // measured and does not help: at ~12 MB in flight the kernel is limited by the DRAM
 // efficiency of sector-granular scattered accesses, not by latency -- profiles/.)
 // Algorithmic bytes per record: 24 (record) + RMW of matched, next_idx,
@@ -122,19 +122,6 @@ __device__ __forceinline__ CellPtrs global_cell_ptrs(const Columns &c, const Rec
     const size_t cell = ok ? static_cast<size_t>(slot) * c.cap + g : 0;
     return CellPtrs{c.matched + cell, c.next_idx + cell, c.peer_committed + cell, c.last_index + (ok ? g : 0),
                     c.pflags + cell};
-}
-
-// Stage 2 of the apply pipeline: pull the record's cell (and its group's meta word) into L2.
-__device__ __forceinline__ void prefetch_cell(const Columns &c, const RecRegs &r) {
-    const uint32_t g = static_cast<uint32_t>(r.w0);
-    const uint32_t slot = static_cast<uint32_t>(r.w0 >> 32) & 0xffu;
-    if (((r.w0 >> 40) & RAFTGPU_REC_EXT) || g >= c.cap || slot >= kSlots) return;
-    const size_t cell = static_cast<size_t>(slot) * c.cap + g;
-    prefetch_l2(c.matched + cell);
-    prefetch_l2(c.next_idx + cell);
-    prefetch_l2(c.peer_committed + cell);
-    prefetch_l2(c.pflags + cell);
-    prefetch_l2(c.meta + g);
 }
 
 __device__ __forceinline__ CellRegs load_cell(const Columns &c, const RecRegs &r) {
@@ -286,7 +273,7 @@ __device__ __forceinline__ uint32_t apply_one(const Columns &c, const void *recs
 // its cell in `touched` ([cap] bytes, one bit per peer slot, cleared by the caller beforehand)
 // with an L2 atomic; a cell marked twice breaks the one-wave precondition -- the record is NOT
 // applied and *dup_count is bumped so the step can fail loudly.
-template <bool kPacked, bool kCheckDup = false, bool kPrefetch = false>
+template <bool kPacked, bool kCheckDup = false>
 __global__ void __launch_bounds__(256, 4)
 apply_kernel(Columns c, const void *__restrict__ recs, uint64_t n, uint8_t *__restrict__ results,
              unsigned long long *__restrict__ counters, uint32_t *__restrict__ touched = nullptr,
@@ -302,7 +289,6 @@ apply_kernel(Columns c, const void *__restrict__ recs, uint64_t n, uint8_t *__re
     CellRegs cell_a = load_cell(c, rec_a);
     for (; i < n; i += stride) {
         const RecRegs rec_c = load_rec<kPacked>(recs, i + 2 * stride, n);  // element k+2: record
-        if (kPrefetch) prefetch_cell(c, rec_c);                    // (optional) its cell -> L2
         const CellRegs cell_b = load_cell(c, rec_b);               // element k+1: cell -> registers
         if constexpr (kCheckDup) {
             const uint32_t g = static_cast<uint32_t>(rec_a.w0), slot = static_cast<uint32_t>(rec_a.w0 >> 32) & 0xffu;

@@ -1,4 +1,4 @@
-// k_recompute.cuh -- the recompute pass: Raft::maybe_commit per group (LDG and TMA feeds).
+// k_recompute.cuh -- the recompute pass: Raft::maybe_commit per group.
 // Part of kernels.cuh (included there, inside namespace raftgpu; not a standalone header).
 
 // ---------------------------------------------------------------------------
@@ -11,7 +11,7 @@
 // Algorithmic bytes per group: 8K (matched) + 4 (meta) + 24 (committed,
 // term_start, last_index) read, 8 written when advanced.
 //
-// Two feeds (LDG, TMA) x two specialisations.  kSimple5 = the host has verified
+// Two specialisations.  kSimple5 = the host has verified
 // from its mirror of the meta column that EVERY group in the range is the plain
 // 5-voter configuration in slots 0..4 (no joint half, no group commit): the
 // kernel then carries no mask logic and no general selection network, which
@@ -133,8 +133,8 @@ __device__ __forceinline__ void publish_tile(uint32_t *adv_bitmap, uint64_t g64,
     local[1] += advanced ? 1u : 0u;
 }
 
-// ---- LDG feed: persistent grid, each warp walks 32-group tiles with a grid stride.
-template <bool kSimple5, bool kPrefetch = false>
+// Persistent grid, each warp walks 32-group tiles with a grid stride.
+template <bool kSimple5>
 __global__ void __launch_bounds__(256, kSimple5 ? 6 : 4)
 recompute_kernel(Columns c, uint32_t first, uint32_t n, uint32_t hint_arg,
                  uint32_t *__restrict__ adv_bitmap, uint64_t *__restrict__ commit_out,
@@ -153,23 +153,6 @@ recompute_kernel(Columns c, uint32_t first, uint32_t n, uint32_t hint_arg,
         const uint64_t g64 = static_cast<uint64_t>(base) + (static_cast<uint64_t>(tile) << 5) + lane;
         const bool active = g64 >= first && g64 < end;
         const uint32_t g = static_cast<uint32_t>(g64);
-        // pull this warp's NEXT tile into L2 while the current one is processed; each row of a tile
-        // is 256 contiguous bytes = two 128-byte lines, so lanes 0..1 cover it (slots by lane / 2)
-        if (kPrefetch && tile + n_warps < n_tiles) {
-            const uint64_t gn = static_cast<uint64_t>(base) + (static_cast<uint64_t>(tile + n_warps) << 5);
-            const uint32_t row = lane >> 1, half = (lane & 1u) * 16u;
-            if (row < kSlots) {
-                if ((hint >> row) & 1u) prefetch_l2(c.matched + static_cast<size_t>(row) * c.cap + gn + half);
-            } else if (row == kSlots) {
-                prefetch_l2(c.committed + gn + half);
-            } else if (row == kSlots + 1) {
-                prefetch_l2(c.term_start + gn + half);
-            } else if (row == kSlots + 2) {
-                prefetch_l2(c.last_index + gn + half);
-            } else if (row == kSlots + 3 && half == 0) {
-                prefetch_l2(c.meta + gn);
-            }
-        }
         bool advanced = false, wide_hi = false;
         if (active) {
             // one batch of independent loads
@@ -196,175 +179,6 @@ recompute_kernel(Columns c, uint32_t first, uint32_t n, uint32_t hint_arg,
         }
         publish_tile(adv_bitmap, g64, lane, active, advanced, local);
         if (wide_hi) local[0]--;  // publish_tile counted the lane as a recompute
-    }
-    const int which[2] = {kCntRecomputes, kCntAdvanced};
-    block_flush_counts<2>(local, which, counters, step_advanced);
-}
-
-// ---- TMA feed.
-// The LDG feed is long-scoreboard bound: the bytes it keeps in flight are capped
-// by registers x occupancy.  Here a producer warp streams whole column tiles into
-// a ring of shared-memory stages with 1-D bulk copies (cp.async.bulk, SASS
-// UBLKCP) that complete on an mbarrier, so up to ~200 KB per SM are in flight
-// whatever the consumer warps are doing; the consumers only touch shared memory
-// and write `committed` back with coalesced stores.
-//
-//   stage layout:  [rows][kTile] u64   rows = hinted matched slots (ascending),
-//                                      then committed, term_start, last_index
-//                  [kTile] u32         meta
-//   full[stage]  : producer arms with expect_tx(bytes); the copies complete it
-//   empty[stage] : one arrival per consumer warp releases the stage
-constexpr int kTile = 512;               // groups per stage = consumer threads
-constexpr int kTmaThreads = kTile + 32;  // + one producer warp
-constexpr int kMaxStages = 12;
-
-__device__ __forceinline__ uint32_t smem_u32(const void *p) {
-    return static_cast<uint32_t>(__cvta_generic_to_shared(p));
-}
-__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes)
-                 : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
-    asm volatile(
-        "{\n\t"
-        ".reg .pred p;\n\t"
-        "WAIT_LOOP:\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
-        "@p bra DONE;\n\t"
-        "bra WAIT_LOOP;\n\t"
-        "DONE:\n\t"
-        "}" ::"r"(smem_u32(bar)),
-        "r"(parity)
-        : "memory");
-}
-// 1-D TMA: global -> shared, completion counted in bytes on `bar`
-__device__ __forceinline__ void tma_load_1d(void *dst, const void *src, uint32_t bytes, uint64_t *bar) {
-    asm volatile(
-        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
-            smem_u32(dst)),
-        "l"(src), "r"(bytes), "r"(smem_u32(bar))
-        : "memory");
-}
-
-template <bool kSimple5>
-__global__ void __launch_bounds__(kTmaThreads, 1)
-recompute_tma_kernel(Columns c, uint32_t first, uint32_t n, uint32_t hint_arg, int n_stages,
-                     uint32_t *__restrict__ adv_bitmap, uint64_t *__restrict__ commit_out,
-                     uint64_t *__restrict__ mci_out, uint8_t *__restrict__ gc_out,
-                     uint32_t *__restrict__ step_advanced, unsigned long long *__restrict__ counters) {
-    extern __shared__ __align__(128) uint8_t smem[];
-    __shared__ __align__(8) uint64_t full_bar[kMaxStages];
-    __shared__ __align__(8) uint64_t empty_bar[kMaxStages];
-
-    const uint32_t hint = kSimple5 ? 0x1fu : hint_arg;
-    const uint32_t n_hint = kSimple5 ? 5u : static_cast<uint32_t>(__popc(hint & 0xffu));
-    const uint32_t rows = n_hint + 3;
-    const uint32_t stage_bytes = rows * kTile * 8 + kTile * 4;
-    const uint32_t base = first - (first % kTile);
-    const uint64_t end = static_cast<uint64_t>(first) + n;
-    const uint32_t n_tiles = static_cast<uint32_t>((end - base + kTile - 1) / kTile);
-    const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < n_stages; s++) {
-            mbar_init(&full_bar[s], 1);
-            mbar_init(&empty_bar[s], kTile / 32);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-
-    uint32_t local[2] = {0, 0};  // recomputes, advanced
-    if (warp == kTile / 32) {
-        // ===== producer warp: lane 0 arms the stage, then one lane per row issues its copy =====
-        // row -> source: rows [0, n_hint) = matched of the r-th hinted slot, then committed,
-        // term_start, last_index, and row `rows` = meta (u32)
-        const uint8_t *src_base = nullptr;
-        uint32_t elem = 8;
-        if (lane < n_hint) {
-            uint32_t seen = 0;
-            for (int s = 0; s < kSlots; s++) {
-                if (!((hint >> s) & 1u)) continue;
-                if (seen == lane)
-                    src_base = reinterpret_cast<const uint8_t *>(c.matched + static_cast<size_t>(s) * c.cap);
-                seen++;
-            }
-        } else if (lane == n_hint) {
-            src_base = reinterpret_cast<const uint8_t *>(c.committed);
-        } else if (lane == n_hint + 1) {
-            src_base = reinterpret_cast<const uint8_t *>(c.term_start);
-        } else if (lane == n_hint + 2) {
-            src_base = reinterpret_cast<const uint8_t *>(c.last_index);
-        } else if (lane == rows) {
-            src_base = reinterpret_cast<const uint8_t *>(c.meta);
-            elem = 4;
-        }
-        uint32_t it = 0;
-        for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, it++) {
-            const int st = it % n_stages;
-            const uint32_t ph = (it / n_stages) & 1u;
-            const uint64_t g0 = static_cast<uint64_t>(base) + static_cast<uint64_t>(tile) * kTile;
-            uint32_t ng = static_cast<uint32_t>(end - g0 < kTile ? end - g0 : kTile);
-            ng = (ng + 3u) & ~3u;  // 16-byte multiples for the u32 row; stays inside the padded stride
-            if (lane == 0) {
-                mbar_wait(&empty_bar[st], ph ^ 1u);  // fresh barrier: the parity-1 wait passes at once
-                mbar_expect_tx(&full_bar[st], rows * ng * 8 + ng * 4);
-            }
-            __syncwarp();
-            if (src_base) {
-                uint8_t *sb = smem + static_cast<size_t>(st) * stage_bytes;
-                tma_load_1d(sb + static_cast<size_t>(lane) * kTile * 8, src_base + g0 * elem, ng * elem,
-                            &full_bar[st]);
-            }
-        }
-    } else {
-        // ===== consumers: one group per thread per tile =====
-        uint32_t it = 0;
-        for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, it++) {
-            const int st = it % n_stages;
-            const uint32_t ph = (it / n_stages) & 1u;
-            const uint64_t g64 = static_cast<uint64_t>(base) + static_cast<uint64_t>(tile) * kTile + threadIdx.x;
-            const bool active = g64 >= first && g64 < end;
-            const uint32_t g = static_cast<uint32_t>(g64);
-            const uint8_t *sb = smem + static_cast<size_t>(st) * stage_bytes;
-            const uint64_t *row = reinterpret_cast<const uint64_t *>(sb) + threadIdx.x;
-            mbar_wait(&full_bar[st], ph);
-            // everything this thread needs from the stage, into registers
-            const uint32_t meta =
-                reinterpret_cast<const uint32_t *>(sb + static_cast<size_t>(rows) * kTile * 8)[threadIdx.x];
-            uint64_t v[kSlots];
-            uint32_t r = 0;
-#pragma unroll
-            for (int s = 0; s < kSlots; s++) {
-                v[s] = 0;
-                if ((hint >> s) & 1u) {
-                    v[s] = row[static_cast<size_t>(r) * kTile];
-                    r++;
-                }
-            }
-            const uint64_t committed = row[static_cast<size_t>(n_hint) * kTile];
-            const uint64_t term_start = row[static_cast<size_t>(n_hint + 1) * kTile];
-            const uint64_t last_index = row[static_cast<size_t>(n_hint + 2) * kTile];
-            // the stage can be refilled as soon as every lane of this warp has its values
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&empty_bar[st]);
-            bool advanced = false;
-            if (active) {
-                uint64_t mci;
-                bool use_gc;
-                eval_mci<kSimple5>(c, g, meta, v, hint, mci, use_gc);
-                advanced = commit_group(c, g, meta, mci, use_gc, committed, term_start, last_index,
-                                        commit_out, mci_out, gc_out);
-            }
-            publish_tile(adv_bitmap, g64, lane, active, advanced, local);
-        }
     }
     const int which[2] = {kCntRecomputes, kCntAdvanced};
     block_flush_counts<2>(local, which, counters, step_advanced);

@@ -10,17 +10,18 @@
 // ordered by group, a tile of kFTile consecutive groups owns a CONTIGUOUS record range, so the
 // whole step becomes dense traffic: per tile the producer warp bulk-loads (TMA, cp.async.bulk)
 // the tile's rows of matched / next_idx / committed_index / pflags / meta / committed /
-// term_start / last_index and its record range into one shared-memory stage; the consumers
-//   A. apply every record of the tile to the shared-memory rows (one thread per record;
+// term_start / last_index into one shared-memory stage; the consumers
+//   A. apply every record of the tile, read straight from HBM / L2, to the shared-memory rows (one thread per record;
 //      distinct cells per wave, so no conflicts),
 //   B. recompute the commit index of the tile's groups from the same shared-memory rows
 //      (matched is read from HBM once per step instead of twice),
 //   C. bulk-store the rows back (cp.async.bulk.global.shared::cta).
 // Peer slots outside `hint` (learners) and the cold columns are handled through HBM directly.
 // tile_off[t] = index of the first packed record of tile t (raftgpu_tile_index builds it).
-constexpr int kFTile = RAFTGPU_TILE_GROUPS;  // groups per tile
-// consumer groups: tile i of a CTA is handled by group i % kNG, so the phases of kNG tiles overlap
-// inside one CTA; each group has kCT threads (kCT >= kFTile).  Template parameters of the kernel.
+constexpr int kFTile = RAFTGPU_TILE_GROUPS;  // groups per tile = threads per consumer group
+// consumer groups per CTA: tile i of a CTA is handled by group i % kFGroups, so the phases of kFGroups tiles overlap
+// inside one CTA (DESIGN 3.4: why three)
+constexpr int kFGroups = 3;
 constexpr int kFMaxStages = 8;
 // Row strides inside a stage.  Records arrive in group order, so the ~3.5 records of one group sit
 // in neighbouring lanes and touch the SAME column index of DIFFERENT rows: with a 256-element row
@@ -30,27 +31,72 @@ constexpr uint32_t kFRow64 = (kFTile + 2) * 8;   // bytes per u64 row
 constexpr uint32_t kFRow8 = kFTile + 16;         // bytes per u8 (pflags) row
 constexpr uint32_t kFDefer = 32;                 // deferred (rare-path) records per warp per tile; more are handled inline
 
-__device__ __forceinline__ void named_bar_sync(int id, int n_threads) {
-    asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n_threads) : "memory");
+__device__ __forceinline__ uint32_t smem_u32(const void *p) {
+    return static_cast<uint32_t>(__cvta_generic_to_shared(p));
 }
-// A consumer's wait for "the loads of MY tile have landed in this stage".  A consumer group sees only every kNG-th
-// tile, so on one stage's `full` barrier it skips phases -- and a parity wait is only exact while the waiter is at
-// most ONE phase ahead.  With uniform tiles that always holds; with a batch that covers only part of the groups it
-// does not (record-less tiles are done in a microsecond, loads of light and heavy tiles land out of order): a group
-// could pass the barrier of a stage still armed for the PREVIOUS tile and work on half-landed rows.  So it first
-// waits for the previous use of the stage to be DONE (`done` barrier, previous phase).  That wait is exact: the
-// group's own previous tile was loaded, hence the tile n_stages before IT was stored, stores happen in tile order,
-// and with n_stages >= kNG that covers the previous user of this stage; and once the previous user is done, the
-// `full` barrier is in this tile's phase, so the second wait is exact too.
-__device__ __forceinline__ void wait_stage(uint64_t *full_bar, uint64_t *done_bar, uint32_t parity) {
-    mbar_wait(done_bar, parity ^ 1u);  // (first use of a stage: the parity-1 wait on a fresh barrier passes at once)
-    mbar_wait(full_bar, parity);
+__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
+    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
+}
+__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes)
+                 : "memory");
+}
+__device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
+    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
+}
+__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
+    asm volatile(
+        "{\n\t"
+        ".reg .pred p;\n\t"
+        "WAIT_LOOP:\n\t"
+        "mbarrier.try_wait.parity.shared::cta.b64 p, [%0], %1;\n\t"
+        "@p bra DONE;\n\t"
+        "bra WAIT_LOOP;\n\t"
+        "DONE:\n\t"
+        "}" ::"r"(smem_u32(bar)),
+        "r"(parity)
+        : "memory");
+}
+// 1-D TMA: global -> shared, completion counted in bytes on `bar`
+__device__ __forceinline__ void tma_load_1d(void *dst, const void *src, uint32_t bytes, uint64_t *bar) {
+    asm volatile(
+        "cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(
+            smem_u32(dst)),
+        "l"(src), "r"(bytes), "r"(smem_u32(bar))
+        : "memory");
 }
 // 1-D TMA store: shared -> global, tracked by the per-thread bulk async-group
 __device__ __forceinline__ void tma_store_1d(void *dst, const void *src, uint32_t bytes) {
     asm volatile("cp.async.bulk.global.shared::cta.bulk_group [%0], [%1], %2;" ::"l"(dst), "r"(smem_u32(src)),
                  "r"(bytes)
                  : "memory");
+}
+__device__ __forceinline__ void named_bar_sync(int id, int n_threads) {
+    asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n_threads) : "memory");
+}
+// A consumer's wait for "the loads of MY tile have landed in this stage".  A consumer group sees only every kFGroups-th
+// tile, so on one stage's `full` barrier it skips phases -- and a parity wait is only exact while the waiter is at
+// most ONE phase ahead.  With uniform tiles that always holds; with a batch that covers only part of the groups it
+// does not (record-less tiles are done in a microsecond, loads of light and heavy tiles land out of order): a group
+// could pass the barrier of a stage still armed for the PREVIOUS tile and work on half-landed rows.  So it first
+// waits for the previous use of the stage to be DONE (`done` barrier, previous phase).  That wait is exact: the
+// group's own previous tile was loaded, hence the tile n_stages before IT was stored, stores happen in tile order,
+// and with n_stages >= kFGroups that covers the previous user of this stage; and once the previous user is done, the
+// `full` barrier is in this tile's phase, so the second wait is exact too.
+__device__ __forceinline__ void wait_stage(uint64_t *full_bar, uint64_t *done_bar, uint32_t parity) {
+    mbar_wait(done_bar, parity ^ 1u);  // (first use of a stage: the parity-1 wait on a fresh barrier passes at once)
+    mbar_wait(full_bar, parity);
+}
+
+// The peer slot of the r-th hinted row of a stage.
+__device__ __forceinline__ uint32_t hinted_slot(uint32_t hint, uint32_t r) {
+    uint32_t slot = 0, seen = 0;
+    for (uint32_t s2 = 0; s2 < kSlots; s2++)
+        if ((hint >> s2) & 1u) {
+            if (seen == r) slot = s2;
+            seen++;
+        }
+    return slot;
 }
 
 struct TileArgs {
@@ -59,7 +105,6 @@ struct TileArgs {
     uint32_t n_groups;         // groups [0, n_groups)
     uint32_t hint;
     int n_stages;
-    uint32_t rec_cap;          // packed records staged per tile (multiple of 4); the rest is read from HBM
     uint8_t *results;          // nullable, one byte per packed record
     uint32_t *adv_bitmap;      // nullable
     uint64_t *commit_out;      // nullable
@@ -70,14 +115,57 @@ struct TileArgs {
 };
 
 // bytes of one stage for H hinted slots (shared by host and device)
-__host__ __device__ constexpr uint32_t tile_stage_bytes(uint32_t H, uint32_t rec_cap) {
-    return 3u * H * kFRow64 + 3u * kFRow64 + kFTile * 4u + H * kFRow8 + rec_cap * 16u;
+__host__ __device__ constexpr uint32_t tile_stage_bytes(uint32_t H) {
+    return 3u * H * kFRow64 + 3u * kFRow64 + kFTile * 4u + H * kFRow8;
 }
 
-template <bool kSimple5, int kCT, int kNG>
-__global__ void __launch_bounds__(kCT *kNG + 64, 1) step_tile_kernel(Columns c, TileArgs a) {
-    static_assert(kCT >= kFTile && kCT % 32 == 0, "a consumer group covers a tile");
-    const uint32_t kFRecCap = a.rec_cap;
+// The store warp of both fused kernels: once the consumers are done with a stage, its rows go back to HBM (and the
+// `committed` row to commit_out as well: one dense copy, not 8-byte scatters), then the stage is free for the load
+// warp.  The stage layout both kernels share: H rows each of matched, next_idx and committed_index, then committed,
+// term_start, last_index, meta, and H pflags rows.  no_stores: diagnostics only (RAFTGPU_TILE_SKIP, results are WRONG).
+__device__ __forceinline__ void tile_store_warp(const Columns &c, uint8_t *smem, uint32_t stage_bytes, uint32_t n_groups,
+                                                uint32_t hint, uint32_t H, int n_stages, uint64_t *commit_out,
+                                                bool no_stores, uint64_t *done_bar, uint64_t *empty_bar) {
+    const uint32_t o_next = H * kFRow64, o_pc = 2u * H * kFRow64, o_committed = 3u * H * kFRow64,
+                   o_li = o_committed + 2u * kFRow64, o_flags = o_committed + 3u * kFRow64 + kFTile * 4u;
+    const uint32_t n_tiles = (n_groups + kFTile - 1) / kFTile;
+    const uint32_t lane = threadIdx.x & 31;
+    const uint32_t n_out = 4u * H + 2u + (commit_out ? 1u : 0u);
+    uint32_t it = 0;
+    for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, it++) {
+        const int st = it % n_stages;
+        const uint32_t ph = (it / n_stages) & 1u;
+        const uint32_t g0 = tile * kFTile;
+        const uint32_t ng = n_groups - g0 < kFTile ? n_groups - g0 : kFTile;
+        const uint32_t ng16 = (ng + 15u) & ~15u;
+        uint8_t *sb = smem + static_cast<size_t>(st) * stage_bytes;
+        mbar_wait(&done_bar[st], ph);  // every lane waits: the barrier's completion orders the consumers' writes
+        for (uint32_t j = lane; j < (no_stores ? 0u : n_out); j += 32) {
+            if (j < 4u * H) {
+                const uint32_t col = j / H, r = j % H;
+                const size_t cell = static_cast<size_t>(hinted_slot(hint, r)) * c.cap + g0;
+                if (col == 0) tma_store_1d(c.matched + cell, sb + r * kFRow64, ng16 * 8u);
+                if (col == 1) tma_store_1d(c.next_idx + cell, sb + o_next + r * kFRow64, ng16 * 8u);
+                if (col == 2) tma_store_1d(c.peer_committed + cell, sb + o_pc + r * kFRow64, ng16 * 8u);
+                if (col == 3) tma_store_1d(c.pflags + cell, sb + o_flags + r * kFRow8, ng16);
+            } else if (j == 4u * H) {
+                tma_store_1d(c.committed + g0, sb + o_committed, ng16 * 8u);
+            } else if (j == 4u * H + 1u) {
+                tma_store_1d(c.last_index + g0, sb + o_li, ng16 * 8u);
+            } else {
+                tma_store_1d(commit_out + g0, sb + o_committed, ng16 * 8u);
+            }
+        }
+        asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+        asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");  // shared memory has been read
+        __syncwarp();
+        if (lane == 0) mbar_arrive(&empty_bar[st]);
+    }
+    asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");  // all stores have landed
+}
+
+template <bool kSimple5>
+__global__ void __launch_bounds__(kFTile *kFGroups + 64, 1) step_tile_kernel(Columns c, TileArgs a) {
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ __align__(8) uint64_t full_bar[kFMaxStages];   // loads landed            (load warp -> consumers)
     __shared__ __align__(8) uint64_t done_bar[kFMaxStages];   // rows final in smem      (consumers -> store warp)
@@ -90,7 +178,7 @@ __global__ void __launch_bounds__(kCT *kNG + 64, 1) step_tile_kernel(Columns c, 
     // stage layout (bytes)
     const uint32_t o_matched = 0, o_next = H * kFRow64, o_pc = 2u * H * kFRow64, o_committed = 3u * H * kFRow64,
                    o_ts = o_committed + kFRow64, o_li = o_ts + kFRow64, o_meta = o_li + kFRow64,
-                   o_flags = o_meta + kFTile * 4u, o_recs = o_flags + H * kFRow8, stage_bytes = tile_stage_bytes(H, a.rec_cap);
+                   o_flags = o_meta + kFTile * 4u, stage_bytes = tile_stage_bytes(H);
     const uint32_t n_tiles = (a.n_groups + kFTile - 1) / kFTile;
     const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
 
@@ -105,81 +193,29 @@ __global__ void __launch_bounds__(kCT *kNG + 64, 1) step_tile_kernel(Columns c, 
     __syncthreads();
 
     uint32_t local[7] = {0, 0, 0, 0, 0, 0, 0};  // records, updates, rejects, decrements, no_progress | recomputes, advanced
-    if (warp == kNG * kCT / 32 + 1) {
-        // ===================== store warp: rows back to HBM, then the stage is free =====================
-        const uint32_t n_out = 4u * H + 2u + (a.commit_out ? 1u : 0u);
-        uint32_t it = 0;
-        for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, it++) {
-            const int st = it % a.n_stages;
-            const uint32_t ph = (it / a.n_stages) & 1u;
-            const uint32_t g0 = tile * kFTile;
-            const uint32_t ng = a.n_groups - g0 < kFTile ? a.n_groups - g0 : kFTile;
-            const uint32_t ng16 = (ng + 15u) & ~15u;
-            uint8_t *sb = smem + static_cast<size_t>(st) * stage_bytes;
-            mbar_wait(&done_bar[st], ph);  // every lane waits: the barrier's completion orders the consumers' writes
-            for (uint32_t j = lane; j < ((a.skip & 4u) ? 0u : n_out); j += 32) {
-                if (j < 4u * H) {
-                    const uint32_t col = j / H, r = j % H;
-                    uint32_t slot = 0, seen = 0;
-                    for (uint32_t s2 = 0; s2 < kSlots; s2++)
-                        if ((hint >> s2) & 1u) {
-                            if (seen == r) slot = s2;
-                            seen++;
-                        }
-                    const size_t cell = static_cast<size_t>(slot) * c.cap + g0;
-                    if (col == 0) tma_store_1d(c.matched + cell, sb + o_matched + r * kFRow64, ng16 * 8u);
-                    if (col == 1) tma_store_1d(c.next_idx + cell, sb + o_next + r * kFRow64, ng16 * 8u);
-                    if (col == 2) tma_store_1d(c.peer_committed + cell, sb + o_pc + r * kFRow64, ng16 * 8u);
-                    if (col == 3) tma_store_1d(c.pflags + cell, sb + o_flags + r * kFRow8, ng16);
-                } else if (j == 4u * H) {
-                    tma_store_1d(c.committed + g0, sb + o_committed, ng16 * 8u);
-                } else if (j == 4u * H + 1u) {
-                    tma_store_1d(c.last_index + g0, sb + o_li, ng16 * 8u);
-                } else {  // the step's commit-index output: the tile's `committed` row, one dense copy (not 8-byte scatters)
-                    tma_store_1d(a.commit_out + g0, sb + o_committed, ng16 * 8u);
-                }
-            }
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-            asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");  // shared memory has been read
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&empty_bar[st]);
-        }
-        asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");  // all stores have landed
-    } else if (warp == kNG * kCT / 32) {
+    if (warp == kFGroups * kFTile / 32 + 1) {
+        tile_store_warp(c, smem, stage_bytes, a.n_groups, hint, H, a.n_stages, a.commit_out, (a.skip & 4u) != 0,
+                        done_bar, empty_bar);
+    } else if (warp == kFGroups * kFTile / 32) {
         // ===================== load warp =====================
-        const uint32_t n_copies = 4u * H + 5u;
+        const uint32_t n_copies = 4u * H + 4u;
         uint32_t it = 0;
-        // the tile index of the NEXT tile is fetched while this one is being issued: a dependent global
-        // load at the top of every iteration would sit on the critical path of the ring
-        uint32_t nx_beg = blockIdx.x < n_tiles ? a.tile_off[blockIdx.x] : 0u, nx_end = blockIdx.x < n_tiles ? a.tile_off[blockIdx.x + 1] : 0u;
         for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, it++) {
             const int st = it % a.n_stages;
             const uint32_t ph = (it / a.n_stages) & 1u;
             const uint32_t g0 = tile * kFTile;
             const uint32_t ng = a.n_groups - g0 < kFTile ? a.n_groups - g0 : kFTile;
             const uint32_t ng16 = (ng + 15u) & ~15u;  // 16-byte multiples for every row; inside the padded stride
-            const uint32_t rbeg = nx_beg, rend = nx_end;
-            if (tile + gridDim.x < n_tiles) {
-                nx_beg = a.tile_off[tile + gridDim.x];
-                nx_end = a.tile_off[tile + gridDim.x + 1];
-            }
-            const uint32_t staged = rend - rbeg < kFRecCap ? rend - rbeg : kFRecCap;
             if (lane == 0) {
                 mbar_wait(&empty_bar[st], ph ^ 1u);
-                mbar_expect_tx(&full_bar[st], 3u * H * ng16 * 8u + H * ng16 + 3u * ng16 * 8u + ng16 * 4u + staged * 16u);
+                mbar_expect_tx(&full_bar[st], 3u * H * ng16 * 8u + H * ng16 + 3u * ng16 * 8u + ng16 * 4u);
             }
             __syncwarp();
             uint8_t *sb = smem + static_cast<size_t>(st) * stage_bytes;
             for (uint32_t j = lane; j < n_copies; j += 32) {
                 if (j < 4u * H) {
                     const uint32_t col = j / H, r = j % H;  // col: 0 matched, 1 next_idx, 2 committed_index, 3 pflags
-                    uint32_t slot = 0, seen = 0;
-                    for (uint32_t s2 = 0; s2 < kSlots; s2++)
-                        if ((hint >> s2) & 1u) {
-                            if (seen == r) slot = s2;
-                            seen++;
-                        }
-                    const size_t cell = static_cast<size_t>(slot) * c.cap + g0;
+                    const size_t cell = static_cast<size_t>(hinted_slot(hint, r)) * c.cap + g0;
                     if (col == 0) tma_load_1d(sb + o_matched + r * kFRow64, c.matched + cell, ng16 * 8u, &full_bar[st]);
                     if (col == 1) tma_load_1d(sb + o_next + r * kFRow64, c.next_idx + cell, ng16 * 8u, &full_bar[st]);
                     if (col == 2) tma_load_1d(sb + o_pc + r * kFRow64, c.peer_committed + cell, ng16 * 8u, &full_bar[st]);
@@ -190,24 +226,22 @@ __global__ void __launch_bounds__(kCT *kNG + 64, 1) step_tile_kernel(Columns c, 
                     tma_load_1d(sb + o_ts, c.term_start + g0, ng16 * 8u, &full_bar[st]);
                 } else if (j == 4u * H + 2) {
                     tma_load_1d(sb + o_li, c.last_index + g0, ng16 * 8u, &full_bar[st]);
-                } else if (j == 4u * H + 3) {
+                } else {
                     tma_load_1d(sb + o_meta, c.meta + g0, ng16 * 4u, &full_bar[st]);
-                } else if (staged) {
-                    tma_load_1d(sb + o_recs, a.recs + rbeg, staged * 16u, &full_bar[st]);
                 }
             }
         }
     } else {
         // ===================== consumers: group cg takes every kFGroups-th tile of this CTA =====================
-        const uint32_t cg = warp / (kCT / 32);
-        const uint32_t tid = threadIdx.x - cg * kCT;
+        const uint32_t cg = warp / (kFTile / 32);
+        const uint32_t tid = threadIdx.x - cg * kFTile;
         const int bar_id = 1 + static_cast<int>(cg);
         constexpr uint32_t R64 = kFRow64 / 8;  // row stride in u64 elements
         uint32_t it = 0;
-        const uint32_t first_tile = blockIdx.x + cg * gridDim.x, tile_step = kNG * gridDim.x;
+        const uint32_t first_tile = blockIdx.x + cg * gridDim.x, tile_step = kFGroups * gridDim.x;
         uint32_t nx_beg = first_tile < n_tiles ? a.tile_off[first_tile] : 0u, nx_end = first_tile < n_tiles ? a.tile_off[first_tile + 1] : 0u;
         it = cg;
-        for (uint32_t tile = first_tile; tile < n_tiles; tile += tile_step, it += kNG) {
+        for (uint32_t tile = first_tile; tile < n_tiles; tile += tile_step, it += kFGroups) {
 
             const int st = it % a.n_stages;
             const uint32_t ph = (it / a.n_stages) & 1u;
@@ -218,7 +252,7 @@ __global__ void __launch_bounds__(kCT *kNG + 64, 1) step_tile_kernel(Columns c, 
                 nx_beg = a.tile_off[tile + tile_step];
                 nx_end = a.tile_off[tile + tile_step + 1];
             }
-            const uint32_t cnt = rend - rbeg, staged = cnt < kFRecCap ? cnt : kFRecCap;
+            const uint32_t cnt = rend - rbeg;
             uint8_t *sb = smem + static_cast<size_t>(st) * stage_bytes;
             uint64_t *s_matched = reinterpret_cast<uint64_t *>(sb + o_matched);
             uint64_t *s_next = reinterpret_cast<uint64_t *>(sb + o_next);
@@ -228,28 +262,24 @@ __global__ void __launch_bounds__(kCT *kNG + 64, 1) step_tile_kernel(Columns c, 
             uint64_t *s_li = reinterpret_cast<uint64_t *>(sb + o_li);
             uint32_t *s_meta = reinterpret_cast<uint32_t *>(sb + o_meta);
             uint8_t *s_flags = sb + o_flags;
-            const PackedRec *s_recs = reinterpret_cast<const PackedRec *>(sb + o_recs);
             const ulonglong2 *g_recs = reinterpret_cast<const ulonglong2 *>(a.recs + rbeg);
-            // direct records: this thread's first record is requested BEFORE the wait for the stage (its address does
+            // this thread's first record is requested BEFORE the wait for the stage (its address does
             // not depend on it); the loop then fetches one record ahead.  (Two ahead measured 11 % SLOWER -- 83.5 vs
             // 75.0 us, scripts/micro_tile.py: the kernel sits at its 72-register ceiling and the consumers are bound by
             // issue latency, not by the record reads.)
             ulonglong2 q_next = make_ulonglong2(kPkExt, 0ull);
-            if (staged == 0 && tid < cnt) q_next = g_recs[tid];
+            if (tid < cnt) q_next = g_recs[tid];
             long long t0 = 0, t1 = 0, t2 = 0, t3 = 0, t4 = 0;
             if (a.dbg && tid == 0) t0 = clock64();
             wait_stage(&full_bar[st], &done_bar[st], ph);
             if (a.dbg && tid == 0) t1 = clock64();
 
             // ---- A: the tile's records against the shared-memory rows (raft.rs:1663-1743)
-            // Records come from the stage when they were staged (rec_cap > 0), else straight from HBM /
-            // L2 (rec_cap == 0: the stage holds rows only, which buys a fifth stage; the records of a
-            // tile were prefetched into L2 while the previous tile was processed, and the loop fetches
-            // the records two iterations ahead).
+            // Records are read straight from HBM / L2: the stage holds rows only, which buys a fifth stage (staging
+            // the records too measured equal, DESIGN 3.4); the records of a tile were prefetched into L2 while the
+            // previous tile was processed, and the loop fetches each record one iteration ahead.
             auto rec_at = [&](uint32_t j) -> ulonglong2 {
-                if (j < staged) return reinterpret_cast<const ulonglong2 *>(s_recs)[j];
-                if (j < cnt) return g_recs[j];
-                return make_ulonglong2(kPkExt, 0ull);
+                return j < cnt ? g_recs[j] : make_ulonglong2(kPkExt, 0ull);
             };
             // The main loop handles the records that make up ~98 % of the traffic -- an accept or a leader-local
             // record for a staged cell of a peer in Replicate or Probe state -- straight on the packed words and the
@@ -323,11 +353,9 @@ __global__ void __launch_bounds__(kCT *kNG + 64, 1) step_tile_kernel(Columns c, 
                         }
                     }
                 }
-                // General path: from the stage when the whole tile is staged, else from HBM.
-                const bool from_smem = staged == cnt;
-                const void *base = from_smem ? static_cast<const void *>(s_recs) : static_cast<const void *>(a.recs + rbeg);
-                const uint64_t nn = from_smem ? staged : cnt;
-                const RecRegs rec = load_rec<true>(base, k, nn);
+                // General path.
+                const PackedRec *base = a.recs + rbeg;
+                const RecRegs rec = load_rec<true>(base, k, cnt);
                 uint32_t res = 0;
                 if (!((rec.w0 >> 40) & RAFTGPU_REC_EXT)) {
                     const uint32_t g2 = static_cast<uint32_t>(rec.w0), slot2 = static_cast<uint32_t>(rec.w0 >> 32) & 0xffu;
@@ -346,21 +374,20 @@ __global__ void __launch_bounds__(kCT *kNG + 64, 1) step_tile_kernel(Columns c, 
                         cd.peer_committed = s_pc[r * R64 + gl2];
                         const CellPtrs sp{&s_matched[r * R64 + gl2], &s_next[r * R64 + gl2], &s_pc[r * R64 + gl2], &s_li[gl2],
                                           &s_flags[r * kFRow8 + gl2]};
-                        res = apply_one<1>(c, base, nn, k, rec, cd, sp, local);
+                        res = apply_one<1>(c, base, cnt, k, rec, cd, sp, local);
                     } else {  // a peer slot outside the hint (a learner): its cell lives in HBM
                         CellRegs cd = load_cell(c, rec);
                         cd.meta = s_meta[gl2];
                         CellPtrs gp = global_cell_ptrs(c, rec);
                         gp.last_index = &s_li[gl2];
-                        res = apply_one<1>(c, base, nn, k, rec, cd, gp, local);
+                        res = apply_one<1>(c, base, cnt, k, rec, cd, gp, local);
                     }
                 }
                 if (a.results) a.results[rbeg + k] = static_cast<uint8_t>(res);
             };
-            if (staged != 0) q_next = rec_at(tid);
-            for (uint32_t k = tid; k < ((a.skip & 1u) ? 0u : cnt); k += kCT) {
+            for (uint32_t k = tid; k < ((a.skip & 1u) ? 0u : cnt); k += kFTile) {
                 const ulonglong2 q = q_next;
-                q_next = rec_at(k + kCT);
+                q_next = rec_at(k + kFTile);
                 const uint64_t w0 = q.x;
                 if (w0 & kPkExt) {
                     if (a.results) a.results[rbeg + k] = 0;
@@ -424,11 +451,11 @@ __global__ void __launch_bounds__(kCT *kNG + 64, 1) step_tile_kernel(Columns c, 
                 const uint32_t nd = s_ndefer[warp] < kFDefer ? s_ndefer[warp] : kFDefer;
                 for (uint32_t j = lane; j < nd; j += 32) slow_record(my_defer[j]);
             }
-            named_bar_sync(bar_id, kCT);
+            named_bar_sync(bar_id, kFTile);
             if (a.dbg && tid == 0) t2 = clock64();
 
             // ---- B: Raft::maybe_commit for the tile's groups (raft.rs:893-904)
-            if (tid < kFTile && !(a.skip & 2u)) {  // warp-uniform: kFTile is a multiple of 32
+            if (!(a.skip & 2u)) {
                 const uint32_t gl = tid;
                 const bool active = gl < ng;
                 const uint32_t g = g0 + gl;
@@ -468,12 +495,12 @@ __global__ void __launch_bounds__(kCT *kNG + 64, 1) step_tile_kernel(Columns c, 
 
             // ---- C: hand the stage to the store warp (generic writes -> async proxy: fence, then signal)
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            named_bar_sync(bar_id, kCT);
+            named_bar_sync(bar_id, kFTile);
             if (a.dbg && tid == 0) t3 = clock64();
             if (tid == 0) mbar_arrive(&done_bar[st]);
-            if (kFRecCap == 0 && tile + tile_step < n_tiles) {  // direct records: next tile's range -> L2 (one line = 8 records)
+            if (tile + tile_step < n_tiles) {  // next tile's record range -> L2 (one line = 8 records)
                 const uint32_t nn = nx_end - nx_beg;
-                for (uint32_t k = tid * 8u; k < nn; k += kCT * 8u) prefetch_l2(a.recs + nx_beg + k);
+                for (uint32_t k = tid * 8u; k < nn; k += kFTile * 8u) prefetch_l2(a.recs + nx_beg + k);
             }
             if (a.dbg && tid == 0) {
                 t4 = clock64();

@@ -21,7 +21,6 @@ struct CTileArgs {
     uint32_t n_groups;
     uint32_t hint;
     int n_stages;
-    uint32_t unit_cap;         // units staged in shared memory per tile (multiple of 4); the rest is read from HBM
     uint8_t *results;          // nullable, one byte per unit
     uint32_t *adv_bitmap;      // nullable
     uint64_t *commit_out;      // nullable
@@ -31,12 +30,13 @@ struct CTileArgs {
     uint32_t *dup_count;       // nullable (!kOrdered): bumped for a second record on one cell, which is not applied
 };
 
-__host__ __device__ constexpr uint32_t ctile_stage_bytes(uint32_t H, uint32_t unit_cap) {
-    return 3u * H * kFRow64 + 3u * kFRow64 + kFTile * 4u + H * kFRow8 + unit_cap * 4u;
-}
+// units staged in shared memory per tile (a multiple of 4); the rest of a crowded tile is read from HBM
+constexpr uint32_t kCUnitCap = 1536;
+// a stage: step_tile_kernel's rows, then the tile's units
+__host__ __device__ constexpr uint32_t ctile_stage_bytes(uint32_t H) { return tile_stage_bytes(H) + kCUnitCap * 4u; }
 // dynamic shared memory: the stages, then one u32 run index per group per consumer group
-__host__ __device__ constexpr uint32_t ctile_smem_bytes(uint32_t H, uint32_t unit_cap, int stages, int n_groups_c) {
-    return static_cast<uint32_t>(stages) * ctile_stage_bytes(H, unit_cap) + static_cast<uint32_t>(n_groups_c) * kFTile * 4u;
+__host__ __device__ constexpr uint32_t ctile_smem_bytes(uint32_t H, int stages) {
+    return static_cast<uint32_t>(stages) * ctile_stage_bytes(H) + static_cast<uint32_t>(kFGroups) * kFTile * 4u;
 }
 
 struct TileRows {
@@ -147,9 +147,8 @@ __device__ __forceinline__ bool tile_fast_apply(const Columns &c, const TileRows
 // kOrdered: per-group walk (records of a cell apply in stream order; any number per cell).
 // !kOrdered: one thread per unit (faster; at most one record per (group, peer) cell per batch --
 // checked on the fly in a shared-memory bitmap when a.dup_count is given).
-template <bool kSimple5, int kNG, bool kOrdered>
-__global__ void __launch_bounds__(kFTile *kNG + 64, 1) step_tile_compact_kernel(Columns c, CTileArgs a) {
-    constexpr int kCT = kFTile;
+template <bool kSimple5, bool kOrdered>
+__global__ void __launch_bounds__(kFTile *kFGroups + 64, 1) step_tile_compact_kernel(Columns c, CTileArgs a) {
     extern __shared__ __align__(128) uint8_t smem[];
     __shared__ __align__(8) uint64_t full_bar[kFMaxStages];
     __shared__ __align__(8) uint64_t done_bar[kFMaxStages];
@@ -160,7 +159,7 @@ __global__ void __launch_bounds__(kFTile *kNG + 64, 1) step_tile_compact_kernel(
     const uint32_t o_matched = 0, o_next = H * kFRow64, o_pc = 2u * H * kFRow64, o_committed = 3u * H * kFRow64,
                    o_ts = o_committed + kFRow64, o_li = o_ts + kFRow64, o_meta = o_li + kFRow64,
                    o_flags = o_meta + kFTile * 4u, o_units = o_flags + H * kFRow8,
-                   stage_bytes = ctile_stage_bytes(H, a.unit_cap);
+                   stage_bytes = ctile_stage_bytes(H);
     const uint32_t n_tiles = (a.n_groups + kFTile - 1) / kFTile;
     const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     uint32_t *s_run_all = reinterpret_cast<uint32_t *>(smem + static_cast<size_t>(a.n_stages) * stage_bytes);
@@ -173,51 +172,13 @@ __global__ void __launch_bounds__(kFTile *kNG + 64, 1) step_tile_compact_kernel(
         }
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
-    if (threadIdx.x < kNG * kCT) s_run_all[threadIdx.x] = kOrdered ? 0xffffffffu : 0u;
+    if (threadIdx.x < kFGroups * kFTile) s_run_all[threadIdx.x] = kOrdered ? 0xffffffffu : 0u;
     __syncthreads();
 
     uint32_t local[7] = {0, 0, 0, 0, 0, 0, 0};  // records, updates, rejects, decrements, no_progress | recomputes, advanced
-    if (warp == kNG * kCT / 32 + 1) {
-        // ===================== store warp =====================
-        const uint32_t n_out = 4u * H + 2u + (a.commit_out ? 1u : 0u);
-        uint32_t it = 0;
-        for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, it++) {
-            const int st = it % a.n_stages;
-            const uint32_t ph = (it / a.n_stages) & 1u;
-            const uint32_t g0 = tile * kFTile;
-            const uint32_t ng = a.n_groups - g0 < kFTile ? a.n_groups - g0 : kFTile;
-            const uint32_t ng16 = (ng + 15u) & ~15u;
-            uint8_t *sb = smem + static_cast<size_t>(st) * stage_bytes;
-            mbar_wait(&done_bar[st], ph);
-            for (uint32_t j = lane; j < n_out; j += 32) {
-                if (j < 4u * H) {
-                    const uint32_t col = j / H, r = j % H;
-                    uint32_t slot = 0, seen = 0;
-                    for (uint32_t s2 = 0; s2 < kSlots; s2++)
-                        if ((hint >> s2) & 1u) {
-                            if (seen == r) slot = s2;
-                            seen++;
-                        }
-                    const size_t cell = static_cast<size_t>(slot) * c.cap + g0;
-                    if (col == 0) tma_store_1d(c.matched + cell, sb + o_matched + r * kFRow64, ng16 * 8u);
-                    if (col == 1) tma_store_1d(c.next_idx + cell, sb + o_next + r * kFRow64, ng16 * 8u);
-                    if (col == 2) tma_store_1d(c.peer_committed + cell, sb + o_pc + r * kFRow64, ng16 * 8u);
-                    if (col == 3) tma_store_1d(c.pflags + cell, sb + o_flags + r * kFRow8, ng16);
-                } else if (j == 4u * H) {
-                    tma_store_1d(c.committed + g0, sb + o_committed, ng16 * 8u);
-                } else if (j == 4u * H + 1u) {
-                    tma_store_1d(c.last_index + g0, sb + o_li, ng16 * 8u);
-                } else {  // the step's commit-index output: the tile's `committed` row, one dense copy (not 8-byte scatters)
-                    tma_store_1d(a.commit_out + g0, sb + o_committed, ng16 * 8u);
-                }
-            }
-            asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-            asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-            __syncwarp();
-            if (lane == 0) mbar_arrive(&empty_bar[st]);
-        }
-        asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
-    } else if (warp == kNG * kCT / 32) {
+    if (warp == kFGroups * kFTile / 32 + 1) {
+        tile_store_warp(c, smem, stage_bytes, a.n_groups, hint, H, a.n_stages, a.commit_out, false, done_bar, empty_bar);
+    } else if (warp == kFGroups * kFTile / 32) {
         // ===================== load warp =====================
         const uint32_t n_copies = 4u * H + 5u;
         uint32_t it = 0;
@@ -236,7 +197,7 @@ __global__ void __launch_bounds__(kFTile *kNG + 64, 1) step_tile_compact_kernel(
             }
             const uint32_t ua = u0 & ~3u;
             const uint32_t cnt4 = (u1 - ua + 3u) & ~3u;
-            const uint32_t staged = u1 > u0 ? (cnt4 < a.unit_cap ? cnt4 : a.unit_cap) : 0u;
+            const uint32_t staged = u1 > u0 ? (cnt4 < kCUnitCap ? cnt4 : kCUnitCap) : 0u;
             if (lane == 0) {
                 mbar_wait(&empty_bar[st], ph ^ 1u);
                 mbar_expect_tx(&full_bar[st], 3u * H * ng16 * 8u + H * ng16 + 3u * ng16 * 8u + ng16 * 4u + staged * 4u);
@@ -246,13 +207,7 @@ __global__ void __launch_bounds__(kFTile *kNG + 64, 1) step_tile_compact_kernel(
             for (uint32_t j = lane; j < n_copies; j += 32) {
                 if (j < 4u * H) {
                     const uint32_t col = j / H, r = j % H;
-                    uint32_t slot = 0, seen = 0;
-                    for (uint32_t s2 = 0; s2 < kSlots; s2++)
-                        if ((hint >> s2) & 1u) {
-                            if (seen == r) slot = s2;
-                            seen++;
-                        }
-                    const size_t cell = static_cast<size_t>(slot) * c.cap + g0;
+                    const size_t cell = static_cast<size_t>(hinted_slot(hint, r)) * c.cap + g0;
                     if (col == 0) tma_load_1d(sb + o_matched + r * kFRow64, c.matched + cell, ng16 * 8u, &full_bar[st]);
                     if (col == 1) tma_load_1d(sb + o_next + r * kFRow64, c.next_idx + cell, ng16 * 8u, &full_bar[st]);
                     if (col == 2) tma_load_1d(sb + o_pc + r * kFRow64, c.peer_committed + cell, ng16 * 8u, &full_bar[st]);
@@ -272,15 +227,15 @@ __global__ void __launch_bounds__(kFTile *kNG + 64, 1) step_tile_compact_kernel(
         }
     } else {
         // ===================== consumers: thread gl of group cg owns group g0 + gl of its tiles =====================
-        const uint32_t cg = warp / (kCT / 32);
-        const uint32_t tid = threadIdx.x - cg * kCT;
+        const uint32_t cg = warp / (kFTile / 32);
+        const uint32_t tid = threadIdx.x - cg * kFTile;
         const int bar_id = 1 + static_cast<int>(cg);
         constexpr uint32_t R64 = kFRow64 / 8;
         uint32_t *s_run = s_run_all + cg * kFTile;
         uint32_t it = 0;
         // tile index and g_base words of this consumer group's NEXT tile are fetched during the current
         // one (tile_gb[t] = the g_base words of the two unit blocks tile t starts in)
-        const uint32_t first_tile = blockIdx.x + cg * gridDim.x, tile_step = kNG * gridDim.x;
+        const uint32_t first_tile = blockIdx.x + cg * gridDim.x, tile_step = kFGroups * gridDim.x;
         uint32_t nx_u0 = 0, nx_u1 = 0;
         uint2 nx_gb = make_uint2(0u, 0u);
         if (first_tile < n_tiles) {
@@ -289,7 +244,7 @@ __global__ void __launch_bounds__(kFTile *kNG + 64, 1) step_tile_compact_kernel(
             nx_gb = a.tile_gb[first_tile];
         }
         it = cg;
-        for (uint32_t tile = first_tile; tile < n_tiles; tile += tile_step, it += kNG) {
+        for (uint32_t tile = first_tile; tile < n_tiles; tile += tile_step, it += kFGroups) {
 
             const int st = it % a.n_stages;
             const uint32_t ph = (it / a.n_stages) & 1u;
@@ -305,7 +260,7 @@ __global__ void __launch_bounds__(kFTile *kNG + 64, 1) step_tile_compact_kernel(
             const uint32_t ua = u0 & ~3u;
             const uint32_t lead = u0 - ua, cnt = u1 - ua;  // local unit positions [lead, cnt)
             const uint32_t cnt4 = (cnt + 3u) & ~3u;
-            const uint32_t staged = u1 > u0 ? (cnt4 < a.unit_cap ? cnt4 : a.unit_cap) : 0u;
+            const uint32_t staged = u1 > u0 ? (cnt4 < kCUnitCap ? cnt4 : kCUnitCap) : 0u;
             uint8_t *sb = smem + static_cast<size_t>(st) * stage_bytes;
             TileRows t;
             t.matched = reinterpret_cast<uint64_t *>(sb + o_matched);
@@ -335,7 +290,7 @@ __global__ void __launch_bounds__(kFTile *kNG + 64, 1) step_tile_compact_kernel(
             const bool active = gl < ng;
             const uint32_t g = g0 + gl;
             if constexpr (kOrdered) {
-                for (uint32_t p = lead + tid; p < cnt; p += kCT) {
+                for (uint32_t p = lead + tid; p < cnt; p += kFTile) {
                     const uint32_t u = p < staged ? s_units[p] : g_units[p];
                     const uint32_t kind = u & 3u;
                     if (kind == kCuEsc) {  // a side-table record: start pulling it towards L1 for the walk below
@@ -352,7 +307,7 @@ __global__ void __launch_bounds__(kFTile *kNG + 64, 1) step_tile_compact_kernel(
                     const uint32_t gt = group_of(p, hb) - g0;
                     if (gt < ng) atomicMin(&s_run[gt], p);
                 }
-                named_bar_sync(bar_id, kCT);
+                named_bar_sync(bar_id, kFTile);
                 if (a.dbg && tid == 0) t2 = clock64();
 
                 // ---- 1: the runs of group g, record by record (raft.rs:1663-1743)
@@ -433,7 +388,7 @@ __global__ void __launch_bounds__(kFTile *kNG + 64, 1) step_tile_compact_kernel(
             } else {
                 // ---- 1': one thread per unit; a record finds its run header `back` units behind it
                 uint32_t *s_touch = s_run;  // 2048 bits: (group, peer slot) cells seen in this tile
-                for (uint32_t k = lead + tid; k < cnt; k += kCT) {
+                for (uint32_t k = lead + tid; k < cnt; k += kFTile) {
                     const uint32_t u = k < staged ? s_units[k] : g_units[k];
                     const uint32_t kind = u & 3u;
                     if (kind == kCuHdrA || kind == kCuHdrB) continue;
@@ -497,7 +452,7 @@ __global__ void __launch_bounds__(kFTile *kNG + 64, 1) step_tile_compact_kernel(
                     }
                     if (a.results) a.results[ua + k] = static_cast<uint8_t>(res);
                 }
-                named_bar_sync(bar_id, kCT);
+                named_bar_sync(bar_id, kFTile);
                 if (a.dup_count && tid < kFTile / 4) s_touch[tid] = 0;  // clean for this consumer group's next tile
                 if (a.dbg && tid == 0) t2 = clock64();
             }
@@ -542,7 +497,7 @@ __global__ void __launch_bounds__(kFTile *kNG + 64, 1) step_tile_compact_kernel(
 
             // ---- 3: hand the stage to the store warp
             asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            named_bar_sync(bar_id, kCT);
+            named_bar_sync(bar_id, kFTile);
             if (tid == 0) mbar_arrive(&done_bar[st]);
             if (a.dbg && tid == 0) {
                 t4 = clock64();

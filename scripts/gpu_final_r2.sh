@@ -11,7 +11,7 @@ timeout 300 ncu --set full --clock-control none --import-source on -k regex:step
 timeout 300 ncu --set full --clock-control none --import-source on -k regex:recompute_kernel -s 4 -c 1 -f -o $OUT/prof_recompute python scripts/micro_recompute.py > $OUT/ncu_recompute.log 2>&1
 timeout 300 ncu --set full --clock-control none --import-source on -k regex:wire_ -c 2 -f -o $OUT/prof_wire python scripts/micro_wire.py > $OUT/ncu_wire.log 2>&1
 timeout 400 ncu --set full --clock-control none --import-source on -k regex:tile_compact -s 8 -c 1 -f -o $OUT/prof_compact python bench.py --steps 3 --warmup 3 --e2e-steps 12 --no-sublegs --no-cpu-baseline > $OUT/ncu_compact.log 2>&1
-for k in step_tile_kernel step_tile_compact recompute_tma_kernel; do
+for k in step_tile_kernel step_tile_compact; do
   echo "== $k"; cuobjdump -sass raft-rs_b200/libraftgpu.so 2>/dev/null | awk -v k="$k" '/Function :/{on=index($0,k)>0} on' | grep -oE "UBLKCP[.A-Z0-9]*|SYNCS[.A-Z0-9]*|REDUX[.A-Z0-9]*|UTMA[.A-Z0-9]*|BAR[.A-Z0-9]*|MEMBAR[.A-Z0-9]*|FENCE[.A-Z0-9]*|CCTL[.A-Z0-9]*" | sort | uniq -c | sort -rn | head -20
 done > $OUT/sass_summary.txt 2>&1
 for w in cfg3 cfg4 cfg5; do

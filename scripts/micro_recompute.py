@@ -23,4 +23,4 @@ with torch.cuda.stream(st):
     e1.record(st); torch.cuda.synchronize()
 us = 1e3 * e0.elapsed_time(e1) / (reps * A)
 k = 7 if joint else 5
-print(f"recompute n={n} joint={joint} TMA={os.environ.get('RAFTGPU_TMA','0')} general={os.environ.get('RAFTGPU_FORCE_GENERAL','0')}: {us:.2f} us/pass  {n*(8*k+34)/us/1e3:.0f} GB/s alg")
+print(f"recompute n={n} joint={joint}: {us:.2f} us/pass  {n*(8*k+34)/us/1e3:.0f} GB/s alg")

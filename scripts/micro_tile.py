@@ -1,12 +1,12 @@
 """Micro-benchmark of the fused tile kernel (step_tile_kernel): 1M groups x 5 peers, 4 arenas rotated (inputs larger
 than L2), R rounds each, one CUDA graph of all launches, CUDA events.  With RAFTGPU_TILE_DEBUG=1 the kernel's phase
 cycle counters are printed.  CONFIGS="K=V K=V;K=V;..." lists the knob settings to run after the default
-(RAFTGPU_TILE_VARIANT / _STAGES / _RECCAP / _DEBUG / _SKIP), all in this one process."""
+(RAFTGPU_TILE_DEBUG / _SKIP), all in this one process."""
 import importlib, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 
 os.environ["RAFTGPU_TILE_TUNE"] = "1"      # the library re-reads its RAFTGPU_TILE_* knobs on every launch
-KNOBS = ("RAFTGPU_TILE_VARIANT", "RAFTGPU_TILE_RECCAP", "RAFTGPU_TILE_STAGES", "RAFTGPU_TILE_DEBUG", "RAFTGPU_TILE_SKIP")
+KNOBS = ("RAFTGPU_TILE_DEBUG", "RAFTGPU_TILE_SKIP")
 CONFIGS = [{}, {"RAFTGPU_TILE_DEBUG": "1"}] + [dict(kv.split("=") for kv in c.split()) for c in os.environ.get("CONFIGS", "").split(";") if c.strip()]
 
 import numpy as np, torch

@@ -654,8 +654,9 @@ def test_fused_tile_step_vs_oracle(n, joint):
 
 def test_fused_tile_step_learners_group_commit_and_crowded_tiles():
     """Fused kernel corner cases: peers outside the voter hint (learners -> HBM path), group commit
-    groups (general kernel), a tile with more records than the shared-memory staging holds, records
-    whose EXT payloads straddle that boundary, and a record that is not in its tile."""
+    groups (general kernel), a tile crowded with rejections (about 128 per warp: more than the per-warp
+    deferral list holds, so the rest are applied inside the record loop), and a record that is not in
+    its tile."""
     n = 2000
     synth = B.Synth(n, 0x5EED0009)
     cols = synth.initial
@@ -914,24 +915,6 @@ def test_fused_compact_step_corner_cases():
     O.arena_recompute(ref)
     assert_columns_equal(arena.read_columns(n), ref, n, "duplicate refused")
     arena.close()
-
-
-def test_fused_kernels_in_their_other_configurations():
-    """The tuning knobs are read once per process, so the non-default forms of the fused kernels run in
-    a child process: records staged in shared memory by TMA (RAFTGPU_TILE_RECCAP=1024, the earlier
-    default -- including the tile with more records than the staging holds), two consumer groups,
-    and the compact kernel with two consumer groups and a small unit staging."""
-    import subprocess
-    import sys
-    env = dict(os.environ, RAFTGPU_TILE_RECCAP="1024", RAFTGPU_TILE_VARIANT="2562", RAFTGPU_CTILE_GROUPS="2",
-               RAFTGPU_CTILE_UNITCAP="512")
-    here = os.path.dirname(os.path.abspath(__file__))
-    r = subprocess.run([sys.executable, "-m", "pytest", os.path.join(here, "test_gpu_parity.py"), "-m", "gpu", "-x", "-q",
-                        "-k", "fused_tile_step_learners or (fused_tile_step_vs_oracle and 100003) or "
-                              "fused_compact_step_corner or (fused_compact_step_vs_oracle and 70001)"],
-                       env=env, capture_output=True, text=True, timeout=900)
-    assert r.returncode == 0, r.stdout[-3000:] + r.stderr[-2000:]
-    assert " passed" in r.stdout and "failed" not in r.stdout
 
 
 def _random_state(n, rng):
