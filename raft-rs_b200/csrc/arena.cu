@@ -593,16 +593,14 @@ int32_t create(int32_t device, uint32_t max_groups, uint32_t slots, uint32_t n_r
     TRYC(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, apply_kernel<true>, 256, 0));
     a->grid_apply = std::max(1, occ) * a->sm_count;
     a->tile_smem = 227u * 1024u - 5u * 1024u;  // 227 KB per CTA minus the kernels' static shared memory (barriers, deferred lists)
-    TRYC(cudaFuncSetAttribute(step_tile_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(a->tile_smem)));
-    TRYC(cudaFuncSetAttribute(step_tile_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(a->tile_smem)));
-    TRYC(cudaFuncSetAttribute(step_tile_compact_kernel<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                              static_cast<int>(a->tile_smem)));
-    TRYC(cudaFuncSetAttribute(step_tile_compact_kernel<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                              static_cast<int>(a->tile_smem)));
-    TRYC(cudaFuncSetAttribute(step_tile_compact_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                              static_cast<int>(a->tile_smem)));
-    TRYC(cudaFuncSetAttribute(step_tile_compact_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                              static_cast<int>(a->tile_smem)));
+    const void *const tile_kernels[] = {
+        reinterpret_cast<const void *>(step_tile_kernel<false>), reinterpret_cast<const void *>(step_tile_kernel<true>),
+        reinterpret_cast<const void *>(step_tile_compact_kernel<false, false>),
+        reinterpret_cast<const void *>(step_tile_compact_kernel<true, false>),
+        reinterpret_cast<const void *>(step_tile_compact_kernel<false, true>),
+        reinterpret_cast<const void *>(step_tile_compact_kernel<true, true>)};
+    for (const void *k : tile_kernels)
+        TRYC(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(a->tile_smem)));
     TRYC(cudaStreamCreateWithFlags(&a->s_compute, cudaStreamNonBlocking));
     TRYC(cudaStreamCreateWithFlags(&a->s_h2d, cudaStreamNonBlocking));
     TRYC(cudaStreamCreateWithFlags(&a->s_d2h, cudaStreamNonBlocking));

@@ -1,4 +1,6 @@
-// k_tile.cuh -- step_tile_kernel: the fused apply + recompute tile kernel on packed records (the headline kernel).
+// k_tile.cuh -- step_tile_kernel: the fused apply + recompute tile kernel on packed records (the headline kernel), and
+// the machinery it shares with step_tile_compact_kernel (k_tile_compact.cuh): the stage layout, the load and store
+// warps, the barrier set-up, the commit phase, the hand-over, the general record path and the counter flush.
 // Part of kernels.cuh (included there, inside namespace raftgpu; not a standalone header).
 
 // ---------------------------------------------------------------------------
@@ -8,14 +10,14 @@
 // accesses are sector-granular (8 useful bytes per 32-byte sector request, several rows per
 // record), which HBM serves at roughly half the efficiency of dense bursts.  When the batch is
 // ordered by group, a tile of kFTile consecutive groups owns a CONTIGUOUS record range, so the
-// whole step becomes dense traffic: per tile the producer warp bulk-loads (TMA, cp.async.bulk)
+// whole step becomes dense traffic: per tile the load warp (tile_load_warp) bulk-loads (TMA, cp.async.bulk)
 // the tile's rows of matched / next_idx / committed_index / pflags / meta / committed /
-// term_start / last_index into one shared-memory stage; the consumers
+// term_start / last_index into one shared-memory stage (TileStage); the consumers
 //   A. apply every record of the tile, read straight from HBM / L2, to the shared-memory rows (one thread per record;
 //      distinct cells per wave, so no conflicts),
-//   B. recompute the commit index of the tile's groups from the same shared-memory rows
-//      (matched is read from HBM once per step instead of twice),
-//   C. bulk-store the rows back (cp.async.bulk.global.shared::cta).
+//   B. recompute the commit index of the tile's groups from the same shared-memory rows (tile_commit;
+//      matched is read from HBM once per step instead of twice),
+//   C. hand the stage to the store warp (tile_handoff), which bulk-stores the rows back (tile_store_warp).
 // Peer slots outside `hint` (learners) and the cold columns are handled through HBM directly.
 // tile_off[t] = index of the first packed record of tile t (raftgpu_tile_index builds it).
 constexpr int kFTile = RAFTGPU_TILE_GROUPS;  // groups per tile = threads per consumer group
@@ -30,6 +32,8 @@ constexpr int kFMaxStages = 8;
 constexpr uint32_t kFRow64 = (kFTile + 2) * 8;   // bytes per u64 row
 constexpr uint32_t kFRow8 = kFTile + 16;         // bytes per u8 (pflags) row
 constexpr uint32_t kFDefer = 32;                 // deferred (rare-path) records per warp per tile; more are handled inline
+// units step_tile_compact_kernel stages per tile (a multiple of 4); the rest of a crowded tile is read from HBM
+constexpr uint32_t kCUnitCap = 1536;
 
 __device__ __forceinline__ uint32_t smem_u32(const void *p) {
     return static_cast<uint32_t>(__cvta_generic_to_shared(p));
@@ -99,138 +103,298 @@ __device__ __forceinline__ uint32_t hinted_slot(uint32_t hint, uint32_t r) {
     return slot;
 }
 
-struct TileArgs {
-    const PackedRec *recs;     // packed records in group order
-    const uint32_t *tile_off;  // [n_tiles + 1]
+// One stage of the ring, as both fused kernels lay it out: H rows each of matched, next_idx and committed_index (u64,
+// kFRow64 apart, one per hinted peer slot), then the tile's rows of committed, term_start and last_index (u64), meta
+// (u32), and H pflags rows (u8, kFRow8 apart).  tile_stage_bytes(H) is its size; the compact kernel stages its units
+// behind it.
+__host__ __device__ constexpr uint32_t tile_stage_bytes(uint32_t H) {
+    return 3u * H * kFRow64 + 3u * kFRow64 + kFTile * 4u + H * kFRow8;
+}
+struct TileStage {
+    uint64_t *matched, *next, *pc, *committed, *ts, *li;
+    uint32_t *meta;
+    uint8_t *flags;
+    uint32_t *units;  // step_tile_compact_kernel: the tile's staged units
+    __device__ __forceinline__ TileStage(uint8_t *smem, int st, uint32_t stage_bytes, uint32_t H) {
+        uint8_t *sb = smem + static_cast<size_t>(st) * stage_bytes;
+        const uint32_t o_next = H * kFRow64, o_pc = 2u * H * kFRow64, o_committed = 3u * H * kFRow64,
+                       o_ts = o_committed + kFRow64, o_li = o_ts + kFRow64, o_meta = o_li + kFRow64,
+                       o_flags = o_meta + kFTile * 4u;
+        matched = reinterpret_cast<uint64_t *>(sb);
+        next = reinterpret_cast<uint64_t *>(sb + o_next);
+        pc = reinterpret_cast<uint64_t *>(sb + o_pc);
+        committed = reinterpret_cast<uint64_t *>(sb + o_committed);
+        ts = reinterpret_cast<uint64_t *>(sb + o_ts);
+        li = reinterpret_cast<uint64_t *>(sb + o_li);
+        meta = reinterpret_cast<uint32_t *>(sb + o_meta);
+        flags = sb + o_flags;
+        units = reinterpret_cast<uint32_t *>(sb + tile_stage_bytes(H));
+    }
+};
+
+// Row j of a stage and the HBM row it mirrors, for the tile of groups from g0 (ng16 of them, rounded up to 16 bytes
+// for every row; inside the padded stride): j < 4H the hinted rows of matched, next_idx, committed_index and pflags,
+// then committed, last_index, term_start and meta.  The load warp copies all 4H + 4 in; the store warp writes the
+// first 4H + 2 back.
+struct TileRow {
+    void *smem, *hbm;
+    uint32_t bytes;
+};
+__device__ __forceinline__ TileRow tile_row(const Columns &c, const TileStage &s, uint32_t j, uint32_t hint, uint32_t H,
+                                            uint32_t g0, uint32_t ng16) {
+    constexpr uint32_t R64 = kFRow64 / 8;
+    if (j < 4u * H) {
+        const uint32_t col = j / H, r = j % H;
+        const size_t cell = static_cast<size_t>(hinted_slot(hint, r)) * c.cap + g0;
+        if (col == 0) return {s.matched + r * R64, c.matched + cell, ng16 * 8u};
+        if (col == 1) return {s.next + r * R64, c.next_idx + cell, ng16 * 8u};
+        if (col == 2) return {s.pc + r * R64, c.peer_committed + cell, ng16 * 8u};
+        return {s.flags + r * kFRow8, c.pflags + cell, ng16};
+    }
+    if (j == 4u * H) return {s.committed, c.committed + g0, ng16 * 8u};
+    if (j == 4u * H + 1u) return {s.li, c.last_index + g0, ng16 * 8u};
+    if (j == 4u * H + 2u) return {s.ts, c.term_start + g0, ng16 * 8u};
+    return {s.meta, c.meta + g0, ng16 * 4u};
+}
+
+struct TileBarriers {
+    uint64_t full[kFMaxStages];   // loads landed            (load warp -> consumers)
+    uint64_t done[kFMaxStages];   // rows final in smem      (consumers -> store warp)
+    uint64_t empty[kFMaxStages];  // rows read by the stores (store warp -> load warp)
+};
+__device__ __forceinline__ void tile_init_barriers(TileBarriers &bar, int n_stages) {
+    if (threadIdx.x == 0) {
+        for (int s = 0; s < n_stages; s++) {
+            mbar_init(&bar.full[s], 1);
+            mbar_init(&bar.done[s], 1);
+            mbar_init(&bar.empty[s], 1);
+        }
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+}
+
+// What both fused kernels take besides their records.
+struct FusedArgs {
+    const uint32_t *tile_off;  // [n_tiles + 1]: where tile t's records start
     uint32_t n_groups;         // groups [0, n_groups)
     uint32_t hint;
     int n_stages;
-    uint8_t *results;          // nullable, one byte per packed record
+    uint8_t *results;          // nullable, one byte per packed record / compact unit
     uint32_t *adv_bitmap;      // nullable
     uint64_t *commit_out;      // nullable
     uint32_t *step_advanced;   // nullable
     unsigned long long *counters;
     unsigned long long *dbg;   // nullable: [8] cycle totals per phase (diagnostics, RAFTGPU_TILE_DEBUG=1)
+};
+
+struct TileArgs : FusedArgs {
+    const PackedRec *recs;     // packed records in group order
     uint32_t skip;             // diagnostics only (RAFTGPU_TILE_SKIP, results are WRONG): 1 no records, 2 no recompute, 4 no stores
 };
 
-// bytes of one stage for H hinted slots (shared by host and device)
-__host__ __device__ constexpr uint32_t tile_stage_bytes(uint32_t H) {
-    return 3u * H * kFRow64 + 3u * kFRow64 + kFTile * 4u + H * kFRow8;
+// The load warp of both fused kernels: once the store warp has released a stage, the tile's rows (tile_row) and,
+// given `units` (the compact kernel), up to kCUnitCap of its units from the 16-byte boundary below its first one
+// arrive in it by TMA.  The `full` barrier expects the byte total of the same copies.
+__device__ __forceinline__ void tile_load_warp(const Columns &c, const FusedArgs &a, uint8_t *smem, uint32_t stage_bytes,
+                                               uint32_t hint, uint32_t H, TileBarriers &bar, const uint32_t *units) {
+    const uint32_t n_tiles = (a.n_groups + kFTile - 1) / kFTile;
+    const uint32_t lane = threadIdx.x & 31;
+    const uint32_t n_rows = 4u * H + 4u;
+    uint32_t it = 0;
+    uint32_t nx_u0 = 0, nx_u1 = 0;
+    if (units && blockIdx.x < n_tiles) {
+        nx_u0 = a.tile_off[blockIdx.x];
+        nx_u1 = a.tile_off[blockIdx.x + 1];
+    }
+    for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, it++) {
+        const int st = it % a.n_stages;
+        const uint32_t ph = (it / a.n_stages) & 1u;
+        const uint32_t g0 = tile * kFTile;
+        const uint32_t ng = a.n_groups - g0 < kFTile ? a.n_groups - g0 : kFTile;
+        const uint32_t ng16 = (ng + 15u) & ~15u;
+        uint32_t ua = 0, staged = 0;
+        if (units) {
+            const uint32_t u0 = nx_u0, u1 = nx_u1;
+            if (tile + gridDim.x < n_tiles) {  // next tile's index: fetched while this one is being issued
+                nx_u0 = a.tile_off[tile + gridDim.x];
+                nx_u1 = a.tile_off[tile + gridDim.x + 1];
+            }
+            ua = u0 & ~3u;
+            const uint32_t cnt4 = (u1 - ua + 3u) & ~3u;
+            staged = u1 > u0 ? (cnt4 < kCUnitCap ? cnt4 : kCUnitCap) : 0u;
+        }
+        const TileStage s(smem, st, stage_bytes, H);
+        // copy j < n_rows: row j; copy n_rows: the units (read only)
+        const uint32_t n_copies = n_rows + (staged ? 1u : 0u);
+        auto copy = [&](uint32_t j) -> TileRow {
+            return j < n_rows ? tile_row(c, s, j, hint, H, g0, ng16)
+                              : TileRow{s.units, const_cast<uint32_t *>(units + ua), staged * 4u};
+        };
+        uint32_t bytes = 0;
+        for (uint32_t j = lane; j < n_copies; j += 32) bytes += copy(j).bytes;
+        bytes = __reduce_add_sync(0xffffffffu, bytes);
+        if (lane == 0) {
+            mbar_wait(&bar.empty[st], ph ^ 1u);
+            mbar_expect_tx(&bar.full[st], bytes);
+        }
+        __syncwarp();
+        for (uint32_t j = lane; j < n_copies; j += 32) {
+            const TileRow row = copy(j);
+            tma_load_1d(row.smem, row.hbm, row.bytes, &bar.full[st]);
+        }
+    }
 }
 
 // The store warp of both fused kernels: once the consumers are done with a stage, its rows go back to HBM (and the
 // `committed` row to commit_out as well: one dense copy, not 8-byte scatters), then the stage is free for the load
-// warp.  The stage layout both kernels share: H rows each of matched, next_idx and committed_index, then committed,
-// term_start, last_index, meta, and H pflags rows.  no_stores: diagnostics only (RAFTGPU_TILE_SKIP, results are WRONG).
-__device__ __forceinline__ void tile_store_warp(const Columns &c, uint8_t *smem, uint32_t stage_bytes, uint32_t n_groups,
-                                                uint32_t hint, uint32_t H, int n_stages, uint64_t *commit_out,
-                                                bool no_stores, uint64_t *done_bar, uint64_t *empty_bar) {
-    const uint32_t o_next = H * kFRow64, o_pc = 2u * H * kFRow64, o_committed = 3u * H * kFRow64,
-                   o_li = o_committed + 2u * kFRow64, o_flags = o_committed + 3u * kFRow64 + kFTile * 4u;
-    const uint32_t n_tiles = (n_groups + kFTile - 1) / kFTile;
+// warp.  no_stores: diagnostics only (RAFTGPU_TILE_SKIP, results are WRONG).
+__device__ __forceinline__ void tile_store_warp(const Columns &c, const FusedArgs &a, uint8_t *smem, uint32_t stage_bytes,
+                                                uint32_t hint, uint32_t H, bool no_stores, TileBarriers &bar) {
+    const uint32_t n_tiles = (a.n_groups + kFTile - 1) / kFTile;
     const uint32_t lane = threadIdx.x & 31;
-    const uint32_t n_out = 4u * H + 2u + (commit_out ? 1u : 0u);
+    const uint32_t n_out = 4u * H + 2u + (a.commit_out ? 1u : 0u);
     uint32_t it = 0;
     for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, it++) {
-        const int st = it % n_stages;
-        const uint32_t ph = (it / n_stages) & 1u;
+        const int st = it % a.n_stages;
+        const uint32_t ph = (it / a.n_stages) & 1u;
         const uint32_t g0 = tile * kFTile;
-        const uint32_t ng = n_groups - g0 < kFTile ? n_groups - g0 : kFTile;
+        const uint32_t ng = a.n_groups - g0 < kFTile ? a.n_groups - g0 : kFTile;
         const uint32_t ng16 = (ng + 15u) & ~15u;
-        uint8_t *sb = smem + static_cast<size_t>(st) * stage_bytes;
-        mbar_wait(&done_bar[st], ph);  // every lane waits: the barrier's completion orders the consumers' writes
+        const TileStage s(smem, st, stage_bytes, H);
+        mbar_wait(&bar.done[st], ph);  // every lane waits: the barrier's completion orders the consumers' writes
         for (uint32_t j = lane; j < (no_stores ? 0u : n_out); j += 32) {
-            if (j < 4u * H) {
-                const uint32_t col = j / H, r = j % H;
-                const size_t cell = static_cast<size_t>(hinted_slot(hint, r)) * c.cap + g0;
-                if (col == 0) tma_store_1d(c.matched + cell, sb + r * kFRow64, ng16 * 8u);
-                if (col == 1) tma_store_1d(c.next_idx + cell, sb + o_next + r * kFRow64, ng16 * 8u);
-                if (col == 2) tma_store_1d(c.peer_committed + cell, sb + o_pc + r * kFRow64, ng16 * 8u);
-                if (col == 3) tma_store_1d(c.pflags + cell, sb + o_flags + r * kFRow8, ng16);
-            } else if (j == 4u * H) {
-                tma_store_1d(c.committed + g0, sb + o_committed, ng16 * 8u);
-            } else if (j == 4u * H + 1u) {
-                tma_store_1d(c.last_index + g0, sb + o_li, ng16 * 8u);
-            } else {
-                tma_store_1d(commit_out + g0, sb + o_committed, ng16 * 8u);
-            }
+            const TileRow row = j < 4u * H + 2u ? tile_row(c, s, j, hint, H, g0, ng16)
+                                                : TileRow{s.committed, a.commit_out + g0, ng16 * 8u};
+            tma_store_1d(row.hbm, row.smem, row.bytes);
         }
         asm volatile("cp.async.bulk.commit_group;" ::: "memory");
         asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");  // shared memory has been read
         __syncwarp();
-        if (lane == 0) mbar_arrive(&empty_bar[st]);
+        if (lane == 0) mbar_arrive(&bar.empty[st]);
     }
     asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");  // all stores have landed
+}
+
+// A record that is not on a kernel's fast path (Snapshot state, a REJECT / hostile value, a peer slot outside the
+// hint): the literal apply_one against the shared-memory cell, or against HBM for a slot the tile does not stage.
+// kFmt, recs, n, i: where apply_one finds a REJECT's next_probe_index hint and request_snapshot (k_apply.cuh) --
+// behind position i of the packed records (1), or handed in as n and i (2, compact streams).
+template <int kFmt>
+__device__ __forceinline__ uint32_t tile_general_apply(const Columns &c, const RecRegs &rec, const void *recs, uint64_t n,
+                                                       uint64_t i, uint32_t gl, uint32_t hint, const TileStage &t,
+                                                       uint32_t *local) {
+    constexpr uint32_t R64 = kFRow64 / 8;
+    const uint32_t slot = static_cast<uint32_t>(rec.w0 >> 32) & 0xffu;
+    if (slot < kSlots && ((hint >> slot) & 1u)) {
+        const uint32_t r = __popc(hint & ((1u << slot) - 1u));
+        CellRegs cd;
+        cd.meta = t.meta[gl];
+        cd.matched = t.matched[r * R64 + gl];
+        cd.next_idx = t.next[r * R64 + gl];
+        cd.flags = t.flags[r * kFRow8 + gl];
+        cd.peer_committed = t.pc[r * R64 + gl];
+        const CellPtrs sp{&t.matched[r * R64 + gl], &t.next[r * R64 + gl], &t.pc[r * R64 + gl], &t.li[gl],
+                          &t.flags[r * kFRow8 + gl]};
+        return apply_one<kFmt>(c, recs, n, i, rec, cd, sp, local);
+    }
+    CellRegs cd = load_cell(c, rec);
+    cd.meta = t.meta[gl];
+    CellPtrs gp = global_cell_ptrs(c, rec);
+    gp.last_index = &t.li[gl];
+    return apply_one<kFmt>(c, recs, n, i, rec, cd, gp, local);
+}
+
+// Raft::maybe_commit (raft.rs:893-904) for group g = g0 + gl of a tile from its staged rows, by thread gl of the
+// consumer group (all of them call it: the advanced bitmap is published per warp).
+template <bool kSimple5>
+__device__ __forceinline__ void tile_commit(const Columns &c, const TileStage &s, uint32_t gl, uint32_t g, uint32_t ng,
+                                            uint32_t hint, uint32_t lane, uint32_t *adv_bitmap, uint32_t *local) {
+    constexpr uint32_t R64 = kFRow64 / 8;
+    const bool active = gl < ng;
+    bool advanced = false;
+    if (active) {
+        const uint32_t meta = s.meta[gl];
+        uint64_t v[kSlots];
+        uint32_t r = 0;
+#pragma unroll
+        for (int s2 = 0; s2 < kSlots; s2++) {
+            v[s2] = 0;
+            if ((hint >> s2) & 1u) {
+                v[s2] = s.matched[r * R64 + gl];
+                r++;
+            }
+        }
+        uint64_t mci;
+        bool use_gc;
+        eval_mci<kSimple5>(c, g, meta, v, hint, mci, use_gc);
+        advanced = mci > s.committed[gl] && mci >= s.ts[gl] && mci <= s.li[gl];  // raft_log.rs:488
+        if (advanced) {
+            s.committed[gl] = mci;  // (the store warp copies the row to commit_out too)
+            if (meta & RAFTGPU_META_HAS_SELF) {  // raft.rs:896-900
+                const uint32_t self = RAFTGPU_META_SELF(meta);
+                uint64_t *pc = ((hint >> self) & 1u) ? &s.pc[__popc(hint & ((1u << self) - 1u)) * R64 + gl]
+                                                     : &c.peer_committed[static_cast<size_t>(self) * c.cap + g];
+                if (mci > *pc) *pc = mci;
+            }
+        }
+    }
+    uint32_t lc[2] = {0, 0};
+    publish_tile(adv_bitmap, g, lane, active, advanced, lc);
+    local[5] += lc[0];
+    local[6] += lc[1];
+}
+
+// Hand the stage to the store warp: the consumers' generic writes -> async proxy (fence), the whole consumer group
+// done (named barrier), then one arrive on the stage's `done` barrier.
+__device__ __forceinline__ void tile_handoff(uint64_t *done_bar, int bar_id, uint32_t tid) {
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    named_bar_sync(bar_id, kFTile);
+    if (tid == 0) mbar_arrive(done_bar);
+}
+
+// RAFTGPU_TILE_DEBUG=1: thread 0 of a consumer group adds the intervals between its stamps t[0..3] and now to
+// dbg[0..3] (what each kernel's phases are: at its stamps) and counts the tile in dbg[4].
+__device__ __forceinline__ void tile_debug(unsigned long long *dbg, uint32_t tid, const long long (&clk)[4]) {
+    if (dbg && tid == 0) {
+        const long long now = clock64();
+        atomicAdd(&dbg[0], static_cast<unsigned long long>(clk[1] - clk[0]));
+        atomicAdd(&dbg[1], static_cast<unsigned long long>(clk[2] - clk[1]));
+        atomicAdd(&dbg[2], static_cast<unsigned long long>(clk[3] - clk[2]));
+        atomicAdd(&dbg[3], static_cast<unsigned long long>(now - clk[3]));
+        atomicAdd(&dbg[4], 1ull);
+    }
+}
+
+// Every thread's tallies: records, updates, rejects, decrements, no_progress | recomputes, advanced.
+__device__ __forceinline__ void tile_flush(const uint32_t (&local)[7], const FusedArgs &a) {
+    const int which[7] = {kCntRecords, kCntUpdates, kCntRejects, kCntDecrements, kCntNoProgress, kCntRecomputes, kCntAdvanced};
+    block_flush_counts<7>(local, which, a.counters, nullptr);
+    if (a.step_advanced) {
+        const uint32_t w = __reduce_add_sync(0xffffffffu, local[6]);
+        if ((threadIdx.x & 31) == 0 && w) atomicAdd(a.step_advanced, w);
+    }
 }
 
 template <bool kSimple5>
 __global__ void __launch_bounds__(kFTile *kFGroups + 64, 1) step_tile_kernel(Columns c, TileArgs a) {
     extern __shared__ __align__(128) uint8_t smem[];
-    __shared__ __align__(8) uint64_t full_bar[kFMaxStages];   // loads landed            (load warp -> consumers)
-    __shared__ __align__(8) uint64_t done_bar[kFMaxStages];   // rows final in smem      (consumers -> store warp)
-    __shared__ __align__(8) uint64_t empty_bar[kFMaxStages];  // rows read by the stores (store warp -> load warp)
+    __shared__ __align__(8) TileBarriers bar;
     __shared__ uint32_t s_defer[32][kFDefer];                 // per warp: tile-relative indexes of its rare-path records
     __shared__ uint32_t s_ndefer[32];
 
     const uint32_t hint = kSimple5 ? 0x1fu : (a.hint & 0xffu);
     const uint32_t H = kSimple5 ? 5u : static_cast<uint32_t>(__popc(hint));
-    // stage layout (bytes)
-    const uint32_t o_matched = 0, o_next = H * kFRow64, o_pc = 2u * H * kFRow64, o_committed = 3u * H * kFRow64,
-                   o_ts = o_committed + kFRow64, o_li = o_ts + kFRow64, o_meta = o_li + kFRow64,
-                   o_flags = o_meta + kFTile * 4u, stage_bytes = tile_stage_bytes(H);
+    const uint32_t stage_bytes = tile_stage_bytes(H);
     const uint32_t n_tiles = (a.n_groups + kFTile - 1) / kFTile;
     const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < a.n_stages; s++) {
-            mbar_init(&full_bar[s], 1);
-            mbar_init(&done_bar[s], 1);
-            mbar_init(&empty_bar[s], 1);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
+    tile_init_barriers(bar, a.n_stages);
 
     uint32_t local[7] = {0, 0, 0, 0, 0, 0, 0};  // records, updates, rejects, decrements, no_progress | recomputes, advanced
     if (warp == kFGroups * kFTile / 32 + 1) {
-        tile_store_warp(c, smem, stage_bytes, a.n_groups, hint, H, a.n_stages, a.commit_out, (a.skip & 4u) != 0,
-                        done_bar, empty_bar);
+        tile_store_warp(c, a, smem, stage_bytes, hint, H, (a.skip & 4u) != 0, bar);
     } else if (warp == kFGroups * kFTile / 32) {
-        // ===================== load warp =====================
-        const uint32_t n_copies = 4u * H + 4u;
-        uint32_t it = 0;
-        for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, it++) {
-            const int st = it % a.n_stages;
-            const uint32_t ph = (it / a.n_stages) & 1u;
-            const uint32_t g0 = tile * kFTile;
-            const uint32_t ng = a.n_groups - g0 < kFTile ? a.n_groups - g0 : kFTile;
-            const uint32_t ng16 = (ng + 15u) & ~15u;  // 16-byte multiples for every row; inside the padded stride
-            if (lane == 0) {
-                mbar_wait(&empty_bar[st], ph ^ 1u);
-                mbar_expect_tx(&full_bar[st], 3u * H * ng16 * 8u + H * ng16 + 3u * ng16 * 8u + ng16 * 4u);
-            }
-            __syncwarp();
-            uint8_t *sb = smem + static_cast<size_t>(st) * stage_bytes;
-            for (uint32_t j = lane; j < n_copies; j += 32) {
-                if (j < 4u * H) {
-                    const uint32_t col = j / H, r = j % H;  // col: 0 matched, 1 next_idx, 2 committed_index, 3 pflags
-                    const size_t cell = static_cast<size_t>(hinted_slot(hint, r)) * c.cap + g0;
-                    if (col == 0) tma_load_1d(sb + o_matched + r * kFRow64, c.matched + cell, ng16 * 8u, &full_bar[st]);
-                    if (col == 1) tma_load_1d(sb + o_next + r * kFRow64, c.next_idx + cell, ng16 * 8u, &full_bar[st]);
-                    if (col == 2) tma_load_1d(sb + o_pc + r * kFRow64, c.peer_committed + cell, ng16 * 8u, &full_bar[st]);
-                    if (col == 3) tma_load_1d(sb + o_flags + r * kFRow8, c.pflags + cell, ng16, &full_bar[st]);
-                } else if (j == 4u * H) {
-                    tma_load_1d(sb + o_committed, c.committed + g0, ng16 * 8u, &full_bar[st]);
-                } else if (j == 4u * H + 1) {
-                    tma_load_1d(sb + o_ts, c.term_start + g0, ng16 * 8u, &full_bar[st]);
-                } else if (j == 4u * H + 2) {
-                    tma_load_1d(sb + o_li, c.last_index + g0, ng16 * 8u, &full_bar[st]);
-                } else {
-                    tma_load_1d(sb + o_meta, c.meta + g0, ng16 * 4u, &full_bar[st]);
-                }
-            }
-        }
+        tile_load_warp(c, a, smem, stage_bytes, hint, H, bar, nullptr);
     } else {
         // ===================== consumers: group cg takes every kFGroups-th tile of this CTA =====================
         const uint32_t cg = warp / (kFTile / 32);
@@ -253,15 +417,7 @@ __global__ void __launch_bounds__(kFTile *kFGroups + 64, 1) step_tile_kernel(Col
                 nx_end = a.tile_off[tile + tile_step + 1];
             }
             const uint32_t cnt = rend - rbeg;
-            uint8_t *sb = smem + static_cast<size_t>(st) * stage_bytes;
-            uint64_t *s_matched = reinterpret_cast<uint64_t *>(sb + o_matched);
-            uint64_t *s_next = reinterpret_cast<uint64_t *>(sb + o_next);
-            uint64_t *s_pc = reinterpret_cast<uint64_t *>(sb + o_pc);
-            uint64_t *s_committed = reinterpret_cast<uint64_t *>(sb + o_committed);
-            uint64_t *s_ts = reinterpret_cast<uint64_t *>(sb + o_ts);
-            uint64_t *s_li = reinterpret_cast<uint64_t *>(sb + o_li);
-            uint32_t *s_meta = reinterpret_cast<uint32_t *>(sb + o_meta);
-            uint8_t *s_flags = sb + o_flags;
+            const TileStage s(smem, st, stage_bytes, H);
             const ulonglong2 *g_recs = reinterpret_cast<const ulonglong2 *>(a.recs + rbeg);
             // this thread's first record is requested BEFORE the wait for the stage (its address does
             // not depend on it); the loop then fetches one record ahead.  (Two ahead measured 11 % SLOWER -- 83.5 vs
@@ -269,10 +425,10 @@ __global__ void __launch_bounds__(kFTile *kFGroups + 64, 1) step_tile_kernel(Col
             // issue latency, not by the record reads.)
             ulonglong2 q_next = make_ulonglong2(kPkExt, 0ull);
             if (tid < cnt) q_next = g_recs[tid];
-            long long t0 = 0, t1 = 0, t2 = 0, t3 = 0, t4 = 0;
-            if (a.dbg && tid == 0) t0 = clock64();
-            wait_stage(&full_bar[st], &done_bar[st], ph);
-            if (a.dbg && tid == 0) t1 = clock64();
+            long long clk[4] = {0, 0, 0, 0};
+            if (a.dbg && tid == 0) clk[0] = clock64();
+            wait_stage(&bar.full[st], &bar.done[st], ph);
+            if (a.dbg && tid == 0) clk[1] = clock64();
 
             // ---- A: the tile's records against the shared-memory rows (raft.rs:1663-1743)
             // Records are read straight from HBM / L2: the stage holds rows only, which buys a fifth stage (staging
@@ -302,10 +458,10 @@ __global__ void __launch_bounds__(kFTile *kFGroups + 64, 1) step_tile_kernel(Col
                 if (!(w0 & kPkWide) && (w0 & kPkReject) && gl < ng && ((hint >> slot) & 1u)) {
                     const uint32_t r = kSimple5 ? slot : static_cast<uint32_t>(__popc(hint & ((1u << slot) - 1u)));
                     const uint32_t ci = r * R64 + gl;
-                    const uint32_t f0 = s_flags[r * kFRow8 + gl];
+                    const uint32_t f0 = s.flags[r * kFRow8 + gl];
                     const uint32_t state = f0 & RAFTGPU_PF_STATE_MASK;
-                    const bool present = kSimple5 || (((RAFTGPU_META_IN(s_meta[gl]) | RAFTGPU_META_OUT(s_meta[gl]) |
-                                                        RAFTGPU_META_LEARN(s_meta[gl])) >> slot) & 1u);
+                    const bool present = kSimple5 || (((RAFTGPU_META_IN(s.meta[gl]) | RAFTGPU_META_OUT(s.meta[gl]) |
+                                                        RAFTGPU_META_LEARN(s.meta[gl])) >> slot) & 1u);
                     if (present && state != RAFTGPU_STATE_SNAPSHOT) {
                         // its EXT payloads: [kind 1 hint] [kind 2 snapshot request]
                         uint64_t hint_idx = 0;
@@ -318,13 +474,13 @@ __global__ void __launch_bounds__(kFTile *kFGroups + 64, 1) step_tile_kernel(Col
                         if (!snapshot_req) {
                             const uint64_t index = q.y;
                             const uint32_t delta = static_cast<uint32_t>(w0 >> 40);
-                            uint64_t m = s_matched[ci], nx = s_next[ci];
+                            uint64_t m = s.matched[ci], nx = s.next[ci];
                             const uint64_t nx0 = nx;
                             uint32_t f = f0 | RAFTGPU_PF_RECENT_ACTIVE, res = 0;         // raft.rs:1674
                             local[0]++;
                             local[2]++;
                             const uint64_t commit = index - delta;
-                            if (commit > s_pc[ci]) s_pc[ci] = commit;                   // raft.rs:1677
+                            if (commit > s.pc[ci]) s.pc[ci] = commit;                   // raft.rs:1677
                             bool ok;
                             if (state == RAFTGPU_STATE_REPLICATE) {
                                 ok = index > m;                                          // :173-177 stale otherwise
@@ -346,8 +502,8 @@ __global__ void __launch_bounds__(kFTile *kFGroups + 64, 1) step_tile_kernel(Col
                                     nx = m + 1;
                                 }
                             }
-                            if (nx != nx0) s_next[ci] = nx;
-                            if (f != f0) s_flags[r * kFRow8 + gl] = static_cast<uint8_t>(f);
+                            if (nx != nx0) s.next[ci] = nx;
+                            if (f != f0) s.flags[r * kFRow8 + gl] = static_cast<uint8_t>(f);
                             if (a.results) a.results[rbeg + k] = static_cast<uint8_t>(res);
                             return;
                         }
@@ -358,29 +514,13 @@ __global__ void __launch_bounds__(kFTile *kFGroups + 64, 1) step_tile_kernel(Col
                 const RecRegs rec = load_rec<true>(base, k, cnt);
                 uint32_t res = 0;
                 if (!((rec.w0 >> 40) & RAFTGPU_REC_EXT)) {
-                    const uint32_t g2 = static_cast<uint32_t>(rec.w0), slot2 = static_cast<uint32_t>(rec.w0 >> 32) & 0xffu;
-                    const uint32_t gl2 = g2 - g0;
+                    const uint32_t gl2 = static_cast<uint32_t>(rec.w0) - g0;
                     if (gl2 >= ng) {  // not this tile's group: the batch is not in group order / bad index
                         local[0]++;
                         local[4]++;
                         res = RAFTGPU_RES_NO_PROGRESS;
-                    } else if (slot2 < kSlots && ((hint >> slot2) & 1u)) {
-                        const uint32_t r = __popc(hint & ((1u << slot2) - 1u));
-                        CellRegs cd;
-                        cd.meta = s_meta[gl2];
-                        cd.matched = s_matched[r * R64 + gl2];
-                        cd.next_idx = s_next[r * R64 + gl2];
-                        cd.flags = s_flags[r * kFRow8 + gl2];
-                        cd.peer_committed = s_pc[r * R64 + gl2];
-                        const CellPtrs sp{&s_matched[r * R64 + gl2], &s_next[r * R64 + gl2], &s_pc[r * R64 + gl2], &s_li[gl2],
-                                          &s_flags[r * kFRow8 + gl2]};
-                        res = apply_one<1>(c, base, cnt, k, rec, cd, sp, local);
-                    } else {  // a peer slot outside the hint (a learner): its cell lives in HBM
-                        CellRegs cd = load_cell(c, rec);
-                        cd.meta = s_meta[gl2];
-                        CellPtrs gp = global_cell_ptrs(c, rec);
-                        gp.last_index = &s_li[gl2];
-                        res = apply_one<1>(c, base, cnt, k, rec, cd, gp, local);
+                    } else {
+                        res = tile_general_apply<1>(c, rec, base, cnt, k, gl2, hint, s, local);
                     }
                 }
                 if (a.results) a.results[rbeg + k] = static_cast<uint8_t>(res);
@@ -400,10 +540,10 @@ __global__ void __launch_bounds__(kFTile *kFGroups + 64, 1) step_tile_kernel(Col
                 if (!(w0 & (kPkWide | kPkReject)) && gl < ng && ((hint >> slot) & 1u)) {
                     const uint32_t r = kSimple5 ? slot : static_cast<uint32_t>(__popc(hint & ((1u << slot) - 1u)));
                     const uint32_t ci = r * R64 + gl;
-                    const uint32_t f0 = s_flags[r * kFRow8 + gl];
+                    const uint32_t f0 = s.flags[r * kFRow8 + gl];
                     const uint32_t state = f0 & RAFTGPU_PF_STATE_MASK;
-                    const bool present = kSimple5 || (((RAFTGPU_META_IN(s_meta[gl]) | RAFTGPU_META_OUT(s_meta[gl]) |
-                                                        RAFTGPU_META_LEARN(s_meta[gl])) >> slot) & 1u);
+                    const bool present = kSimple5 || (((RAFTGPU_META_IN(s.meta[gl]) | RAFTGPU_META_OUT(s.meta[gl]) |
+                                                        RAFTGPU_META_LEARN(s.meta[gl])) >> slot) & 1u);
                     if (present && state != RAFTGPU_STATE_SNAPSHOT) {
                         // accept / leader-local: maybe_update (progress.rs:138-150), shared by the accept path
                         // (raft.rs:1674-1677, 1724-1730) and the leader-local path (raft.rs:974-991, 1010-1014);
@@ -411,11 +551,11 @@ __global__ void __launch_bounds__(kFTile *kFGroups + 64, 1) step_tile_kernel(Col
                         const uint64_t index = q.y;
                         const uint32_t delta = static_cast<uint32_t>(w0 >> 40);
                         const bool is_local = (w0 & kPkLocal) != 0;
-                        const uint64_t m = s_matched[ci], nx = s_next[ci], pcv = s_pc[ci];
+                        const uint64_t m = s.matched[ci], nx = s.next[ci], pcv = s.pc[ci];
                         local[0]++;
-                        if (is_local && delta != kPkNoCommit) s_li[gl] = index + delta;   // raft.rs:974-991
+                        if (is_local && delta != kPkNoCommit) s.li[gl] = index + delta;   // raft.rs:974-991
                         const uint64_t commit = index - delta;
-                        if (!is_local && commit > pcv) s_pc[ci] = commit;                 // raft.rs:1677
+                        if (!is_local && commit > pcv) s.pc[ci] = commit;                 // raft.rs:1677
                         const bool probe = state == RAFTGPU_STATE_PROBE;
                         const bool need = m < index;
                         const bool old_paused = !is_local && (f0 & (probe ? RAFTGPU_PF_PAUSED : RAFTGPU_PF_INS_FULL)) != 0;
@@ -430,9 +570,9 @@ __global__ void __launch_bounds__(kFTile *kFGroups + 64, 1) step_tile_kernel(Col
                             c.pending_snapshot[static_cast<size_t>(slot) * c.cap + g] = 0;
                         }
                         local[1] += need ? 1u : 0u;
-                        if (need) s_matched[ci] = index;
-                        if (nnx != nx) s_next[ci] = nnx;
-                        if (f != f0) s_flags[r * kFRow8 + gl] = static_cast<uint8_t>(f);
+                        if (need) s.matched[ci] = index;
+                        if (nnx != nx) s.next[ci] = nnx;
+                        if (f != f0) s.flags[r * kFRow8 + gl] = static_cast<uint8_t>(f);
                         if (a.results)
                             a.results[rbeg + k] = static_cast<uint8_t>(need ? (RAFTGPU_RES_OK | (old_paused ? RAFTGPU_RES_OLD_PAUSED : 0u)) : 0u);
                         done = true;
@@ -452,70 +592,21 @@ __global__ void __launch_bounds__(kFTile *kFGroups + 64, 1) step_tile_kernel(Col
                 for (uint32_t j = lane; j < nd; j += 32) slow_record(my_defer[j]);
             }
             named_bar_sync(bar_id, kFTile);
-            if (a.dbg && tid == 0) t2 = clock64();
+            if (a.dbg && tid == 0) clk[2] = clock64();
 
-            // ---- B: Raft::maybe_commit for the tile's groups (raft.rs:893-904)
-            if (!(a.skip & 2u)) {
-                const uint32_t gl = tid;
-                const bool active = gl < ng;
-                const uint32_t g = g0 + gl;
-                bool advanced = false;
-                if (active) {
-                    const uint32_t meta = s_meta[gl];
-                    uint64_t v[kSlots];
-                    uint32_t r = 0;
-#pragma unroll
-                    for (int s2 = 0; s2 < kSlots; s2++) {
-                        v[s2] = 0;
-                        if ((hint >> s2) & 1u) {
-                            v[s2] = s_matched[r * R64 + gl];
-                            r++;
-                        }
-                    }
-                    uint64_t mci;
-                    bool use_gc;
-                    eval_mci<kSimple5>(c, g, meta, v, hint, mci, use_gc);
-                    advanced = mci > s_committed[gl] && mci >= s_ts[gl] && mci <= s_li[gl];  // raft_log.rs:488
-                    if (advanced) {
-                        s_committed[gl] = mci;  // (the store warp copies the row to commit_out too)
-                        if (meta & RAFTGPU_META_HAS_SELF) {  // raft.rs:896-900
-                            const uint32_t self = RAFTGPU_META_SELF(meta);
-                            uint64_t *pc = ((hint >> self) & 1u)
-                                               ? &s_pc[__popc(hint & ((1u << self) - 1u)) * R64 + gl]
-                                               : &c.peer_committed[static_cast<size_t>(self) * c.cap + g];
-                            if (mci > *pc) *pc = mci;
-                        }
-                    }
-                }
-                uint32_t lc[2] = {0, 0};
-                publish_tile(a.adv_bitmap, static_cast<uint64_t>(g0) + gl, lane, active, advanced, lc);
-                local[5] += lc[0];
-                local[6] += lc[1];
-            }
+            // ---- B: Raft::maybe_commit for the tile's groups
+            if (!(a.skip & 2u)) tile_commit<kSimple5>(c, s, tid, g0 + tid, ng, hint, lane, a.adv_bitmap, local);
 
-            // ---- C: hand the stage to the store warp (generic writes -> async proxy: fence, then signal)
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            named_bar_sync(bar_id, kFTile);
-            if (a.dbg && tid == 0) t3 = clock64();
-            if (tid == 0) mbar_arrive(&done_bar[st]);
-            if (tile + tile_step < n_tiles) {  // next tile's record range -> L2 (one line = 8 records)
+            // ---- C: hand the stage to the store warp, then the next tile's record range -> L2 (one line = 8 records)
+            tile_handoff(&bar.done[st], bar_id, tid);
+            if (a.dbg && tid == 0) clk[3] = clock64();
+            if (tile + tile_step < n_tiles) {
                 const uint32_t nn = nx_end - nx_beg;
                 for (uint32_t k = tid * 8u; k < nn; k += kFTile * 8u) prefetch_l2(a.recs + nx_beg + k);
             }
-            if (a.dbg && tid == 0) {
-                t4 = clock64();
-                atomicAdd(&a.dbg[0], static_cast<unsigned long long>(t1 - t0));  // waiting for the TMA loads
-                atomicAdd(&a.dbg[1], static_cast<unsigned long long>(t2 - t1));  // A: records
-                atomicAdd(&a.dbg[2], static_cast<unsigned long long>(t3 - t2));  // B: recompute (+ fence, barrier)
-                atomicAdd(&a.dbg[3], static_cast<unsigned long long>(t4 - t3));  // C: stores + drain
-                atomicAdd(&a.dbg[4], 1ull);                                       // tiles
-            }
+            // dbg: waiting for the TMA loads, A: records, B: recompute (+ fence, barrier), C: stores + drain
+            tile_debug(a.dbg, tid, clk);
         }
     }
-    const int which[7] = {kCntRecords, kCntUpdates, kCntRejects, kCntDecrements, kCntNoProgress, kCntRecomputes, kCntAdvanced};
-    block_flush_counts<7>(local, which, a.counters, nullptr);
-    if (a.step_advanced) {
-        const uint32_t w = __reduce_add_sync(0xffffffffu, local[6]);
-        if (lane == 0 && w) atomicAdd(a.step_advanced, w);
-    }
+    tile_flush(local, a);
 }

@@ -2,82 +2,35 @@
 // Part of kernels.cuh (included there, inside namespace raftgpu; not a standalone header).
 
 // step_tile_compact_kernel: the fused step for a TILEABLE compact stream (groups ascending, every
-// run headed -- raftgpu_compact_hdr.flags & RAFTGPU_COMPACT_TILEABLE).  Same producer / store
-// warps and stage ring as step_tile_kernel; the consumers work per GROUP instead of per record:
+// run headed -- raftgpu_compact_hdr.flags & RAFTGPU_COMPACT_TILEABLE).  Everything but the record
+// loop is step_tile_kernel's (k_tile.cuh): stage ring and layout, load warp (which also stages the
+// tile's units behind the rows), store warp, commit phase, hand-over, general record path and counter
+// flush.  The consumers work per GROUP instead of per record:
 //   0. a unit-parallel pre-pass finds, for every group of the tile, the first unit of its first
 //      run (shared-memory atomicMin on the run headers),
 //   1. thread gl then walks the runs of group g0+gl SEQUENTIALLY -- header decoded once, each
 //      record a handful of instructions against the shared-memory cells -- so the records of one
 //      cell apply in stream order (no one-wave restriction) and
-//   2. goes straight on to the group's Raft::maybe_commit: its cells were written by this very
-//      thread, so no barrier separates apply and recompute.
+//   2. goes straight on to the group's Raft::maybe_commit (tile_commit): its cells were written by
+//      this very thread, so no barrier separates apply and recompute.
 // Against the per-record form this is ~2.5x fewer warp instructions per tile (no per-record
 // header/cell address arithmetic, no three-way divergence on the record kind) and a third of the
 // record bytes.  tile_off[t] = unit position of the first run header of tile t.
-struct CTileArgs {
+struct CTileArgs : FusedArgs {  // (tile_off: unit positions; results: one byte per unit)
     CompactSrc src;
-    const uint32_t *tile_off;  // [n_tiles + 1], unit positions
     const uint2 *tile_gb;      // [n_tiles]: g_base of the unit block tile t starts in, and of the next block
-    uint32_t n_groups;
-    uint32_t hint;
-    int n_stages;
-    uint8_t *results;          // nullable, one byte per unit
-    uint32_t *adv_bitmap;      // nullable
-    uint64_t *commit_out;      // nullable
-    uint32_t *step_advanced;   // nullable
-    unsigned long long *counters;
-    unsigned long long *dbg;   // nullable
     uint32_t *dup_count;       // nullable (!kOrdered): bumped for a second record on one cell, which is not applied
 };
 
-// units staged in shared memory per tile (a multiple of 4); the rest of a crowded tile is read from HBM
-constexpr uint32_t kCUnitCap = 1536;
-// a stage: step_tile_kernel's rows, then the tile's units
-__host__ __device__ constexpr uint32_t ctile_stage_bytes(uint32_t H) { return tile_stage_bytes(H) + kCUnitCap * 4u; }
-// dynamic shared memory: the stages, then one u32 run index per group per consumer group
-__host__ __device__ constexpr uint32_t ctile_smem_bytes(uint32_t H, int stages) {
-    return static_cast<uint32_t>(stages) * ctile_stage_bytes(H) + static_cast<uint32_t>(kFGroups) * kFTile * 4u;
-}
-
-struct TileRows {
-    uint64_t *matched, *next, *pc, *committed, *ts, *li;
-    uint32_t *meta;
-    uint8_t *flags;
-};
-
-// A record that is not on the fast path (Snapshot state, a REJECT / hostile value from the side
-// table, a peer slot outside the hint): the literal apply_one against the shared-memory cell, or
-// against HBM for a slot the tile does not stage.
-__device__ __forceinline__ uint32_t tile_general_apply(const Columns &c, const RecRegs &rec, uint64_t ext_hint,
-                                                    uint64_t ext_snapshot, uint32_t gl, uint32_t hint,
-                                                    const TileRows &t, uint32_t *local) {
-    constexpr uint32_t R64 = kFRow64 / 8;
-    const uint32_t slot = static_cast<uint32_t>(rec.w0 >> 32) & 0xffu;
-    if (slot < kSlots && ((hint >> slot) & 1u)) {
-        const uint32_t r = __popc(hint & ((1u << slot) - 1u));
-        CellRegs cd;
-        cd.meta = t.meta[gl];
-        cd.matched = t.matched[r * R64 + gl];
-        cd.next_idx = t.next[r * R64 + gl];
-        cd.flags = t.flags[r * kFRow8 + gl];
-        cd.peer_committed = t.pc[r * R64 + gl];
-        const CellPtrs sp{&t.matched[r * R64 + gl], &t.next[r * R64 + gl], &t.pc[r * R64 + gl], &t.li[gl],
-                          &t.flags[r * kFRow8 + gl]};
-        return apply_one<2>(c, nullptr, ext_hint, ext_snapshot, rec, cd, sp, local);
-    }
-    CellRegs cd = load_cell(c, rec);
-    cd.meta = t.meta[gl];
-    CellPtrs gp = global_cell_ptrs(c, rec);
-    gp.last_index = &t.li[gl];
-    return apply_one<2>(c, nullptr, ext_hint, ext_snapshot, rec, cd, gp, local);
-}
+// shared memory besides the stages: one u32 run index per group per consumer group
+constexpr uint32_t kCRunBytes = static_cast<uint32_t>(kFGroups) * kFTile * 4u;
 
 // The common records -- accept, leader-local, rejection without a snapshot request -- for a peer
 // in Replicate or Probe state whose cell is staged in shared memory: statement for statement the
 // branches of apply_one (raft.rs:1674-1677, 1709-1730, 974-991, 1010-1014; progress.rs:95-114,
 // 138-157, 168-206).  Returns false (nothing touched) when the record needs the general path.
 template <bool kSimple5>
-__device__ __forceinline__ bool tile_fast_apply(const Columns &c, const TileRows &t, uint32_t gl, uint32_t g, uint32_t slot,
+__device__ __forceinline__ bool tile_fast_apply(const Columns &c, const TileStage &t, uint32_t gl, uint32_t g, uint32_t slot,
                                                 uint64_t index, uint64_t commit, bool is_local, bool is_reject,
                                                 uint64_t ext_hint, uint32_t hint, uint32_t present_mask, uint32_t *local,
                                                 uint32_t &res) {
@@ -150,87 +103,27 @@ __device__ __forceinline__ bool tile_fast_apply(const Columns &c, const TileRows
 template <bool kSimple5, bool kOrdered>
 __global__ void __launch_bounds__(kFTile *kFGroups + 64, 1) step_tile_compact_kernel(Columns c, CTileArgs a) {
     extern __shared__ __align__(128) uint8_t smem[];
-    __shared__ __align__(8) uint64_t full_bar[kFMaxStages];
-    __shared__ __align__(8) uint64_t done_bar[kFMaxStages];
-    __shared__ __align__(8) uint64_t empty_bar[kFMaxStages];
+    __shared__ __align__(8) TileBarriers bar;
 
     const uint32_t hint = kSimple5 ? 0x1fu : (a.hint & 0xffu);
     const uint32_t H = kSimple5 ? 5u : static_cast<uint32_t>(__popc(hint));
-    const uint32_t o_matched = 0, o_next = H * kFRow64, o_pc = 2u * H * kFRow64, o_committed = 3u * H * kFRow64,
-                   o_ts = o_committed + kFRow64, o_li = o_ts + kFRow64, o_meta = o_li + kFRow64,
-                   o_flags = o_meta + kFTile * 4u, o_units = o_flags + H * kFRow8,
-                   stage_bytes = ctile_stage_bytes(H);
+    const uint32_t stage_bytes = tile_stage_bytes(H) + kCUnitCap * 4u;  // the rows, then the tile's units
     const uint32_t n_tiles = (a.n_groups + kFTile - 1) / kFTile;
     const uint32_t warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     uint32_t *s_run_all = reinterpret_cast<uint32_t *>(smem + static_cast<size_t>(a.n_stages) * stage_bytes);
-
-    if (threadIdx.x == 0) {
-        for (int s = 0; s < a.n_stages; s++) {
-            mbar_init(&full_bar[s], 1);
-            mbar_init(&done_bar[s], 1);
-            mbar_init(&empty_bar[s], 1);
-        }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
     if (threadIdx.x < kFGroups * kFTile) s_run_all[threadIdx.x] = kOrdered ? 0xffffffffu : 0u;
-    __syncthreads();
+    tile_init_barriers(bar, a.n_stages);
 
     uint32_t local[7] = {0, 0, 0, 0, 0, 0, 0};  // records, updates, rejects, decrements, no_progress | recomputes, advanced
     if (warp == kFGroups * kFTile / 32 + 1) {
-        tile_store_warp(c, smem, stage_bytes, a.n_groups, hint, H, a.n_stages, a.commit_out, false, done_bar, empty_bar);
+        tile_store_warp(c, a, smem, stage_bytes, hint, H, false, bar);
     } else if (warp == kFGroups * kFTile / 32) {
-        // ===================== load warp =====================
-        const uint32_t n_copies = 4u * H + 5u;
-        uint32_t it = 0;
-        uint32_t nx_u0 = blockIdx.x < n_tiles ? a.tile_off[blockIdx.x] : 0u, nx_u1 = blockIdx.x < n_tiles ? a.tile_off[blockIdx.x + 1] : 0u;
-        for (uint32_t tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, it++) {
-            const int st = it % a.n_stages;
-            const uint32_t ph = (it / a.n_stages) & 1u;
-            const uint32_t g0 = tile * kFTile;
-            const uint32_t ng = a.n_groups - g0 < kFTile ? a.n_groups - g0 : kFTile;
-            const uint32_t ng16 = (ng + 15u) & ~15u;
-            // the tile's units, from the 16-byte boundary below its first one
-            const uint32_t u0 = nx_u0, u1 = nx_u1;
-            if (tile + gridDim.x < n_tiles) {  // next tile's index: fetched while this one is being issued
-                nx_u0 = a.tile_off[tile + gridDim.x];
-                nx_u1 = a.tile_off[tile + gridDim.x + 1];
-            }
-            const uint32_t ua = u0 & ~3u;
-            const uint32_t cnt4 = (u1 - ua + 3u) & ~3u;
-            const uint32_t staged = u1 > u0 ? (cnt4 < kCUnitCap ? cnt4 : kCUnitCap) : 0u;
-            if (lane == 0) {
-                mbar_wait(&empty_bar[st], ph ^ 1u);
-                mbar_expect_tx(&full_bar[st], 3u * H * ng16 * 8u + H * ng16 + 3u * ng16 * 8u + ng16 * 4u + staged * 4u);
-            }
-            __syncwarp();
-            uint8_t *sb = smem + static_cast<size_t>(st) * stage_bytes;
-            for (uint32_t j = lane; j < n_copies; j += 32) {
-                if (j < 4u * H) {
-                    const uint32_t col = j / H, r = j % H;
-                    const size_t cell = static_cast<size_t>(hinted_slot(hint, r)) * c.cap + g0;
-                    if (col == 0) tma_load_1d(sb + o_matched + r * kFRow64, c.matched + cell, ng16 * 8u, &full_bar[st]);
-                    if (col == 1) tma_load_1d(sb + o_next + r * kFRow64, c.next_idx + cell, ng16 * 8u, &full_bar[st]);
-                    if (col == 2) tma_load_1d(sb + o_pc + r * kFRow64, c.peer_committed + cell, ng16 * 8u, &full_bar[st]);
-                    if (col == 3) tma_load_1d(sb + o_flags + r * kFRow8, c.pflags + cell, ng16, &full_bar[st]);
-                } else if (j == 4u * H) {
-                    tma_load_1d(sb + o_committed, c.committed + g0, ng16 * 8u, &full_bar[st]);
-                } else if (j == 4u * H + 1) {
-                    tma_load_1d(sb + o_ts, c.term_start + g0, ng16 * 8u, &full_bar[st]);
-                } else if (j == 4u * H + 2) {
-                    tma_load_1d(sb + o_li, c.last_index + g0, ng16 * 8u, &full_bar[st]);
-                } else if (j == 4u * H + 3) {
-                    tma_load_1d(sb + o_meta, c.meta + g0, ng16 * 4u, &full_bar[st]);
-                } else if (staged) {
-                    tma_load_1d(sb + o_units, a.src.units + ua, staged * 4u, &full_bar[st]);
-                }
-            }
-        }
+        tile_load_warp(c, a, smem, stage_bytes, hint, H, bar, a.src.units);
     } else {
         // ===================== consumers: thread gl of group cg owns group g0 + gl of its tiles =====================
         const uint32_t cg = warp / (kFTile / 32);
         const uint32_t tid = threadIdx.x - cg * kFTile;
         const int bar_id = 1 + static_cast<int>(cg);
-        constexpr uint32_t R64 = kFRow64 / 8;
         uint32_t *s_run = s_run_all + cg * kFTile;
         uint32_t it = 0;
         // tile index and g_base words of this consumer group's NEXT tile are fetched during the current
@@ -261,23 +154,14 @@ __global__ void __launch_bounds__(kFTile *kFGroups + 64, 1) step_tile_compact_ke
             const uint32_t lead = u0 - ua, cnt = u1 - ua;  // local unit positions [lead, cnt)
             const uint32_t cnt4 = (cnt + 3u) & ~3u;
             const uint32_t staged = u1 > u0 ? (cnt4 < kCUnitCap ? cnt4 : kCUnitCap) : 0u;
-            uint8_t *sb = smem + static_cast<size_t>(st) * stage_bytes;
-            TileRows t;
-            t.matched = reinterpret_cast<uint64_t *>(sb + o_matched);
-            t.next = reinterpret_cast<uint64_t *>(sb + o_next);
-            t.pc = reinterpret_cast<uint64_t *>(sb + o_pc);
-            t.committed = reinterpret_cast<uint64_t *>(sb + o_committed);
-            t.ts = reinterpret_cast<uint64_t *>(sb + o_ts);
-            t.li = reinterpret_cast<uint64_t *>(sb + o_li);
-            t.meta = reinterpret_cast<uint32_t *>(sb + o_meta);
-            t.flags = sb + o_flags;
-            const uint32_t *s_units = reinterpret_cast<const uint32_t *>(sb + o_units);
+            const TileStage t(smem, st, stage_bytes, H);
+            const uint32_t *s_units = t.units;
             const uint32_t *g_units = a.src.units + ua;
             const uint32_t blk0 = ua / RAFTGPU_COMPACT_BLOCK;
-            long long t0 = 0, t1 = 0, t2 = 0, t3 = 0, t4 = 0;
-            if (a.dbg && tid == 0) t0 = clock64();
-            wait_stage(&full_bar[st], &done_bar[st], ph);  // (k_tile.cuh: exact although this group skips phases)
-            if (a.dbg && tid == 0) t1 = clock64();
+            long long clk[4] = {0, 0, 0, 0};
+            if (a.dbg && tid == 0) clk[0] = clock64();
+            wait_stage(&bar.full[st], &bar.done[st], ph);  // (k_tile.cuh: exact although this group skips phases)
+            if (a.dbg && tid == 0) clk[1] = clock64();
 
             // ---- 0: first run header of every group of the tile.  The g_base words of the (at most
             // two, unless the tile is crowded) unit blocks the tile spans were fetched before the wait.
@@ -308,7 +192,7 @@ __global__ void __launch_bounds__(kFTile *kFGroups + 64, 1) step_tile_compact_ke
                     if (gt < ng) atomicMin(&s_run[gt], p);
                 }
                 named_bar_sync(bar_id, kFTile);
-                if (a.dbg && tid == 0) t2 = clock64();
+                if (a.dbg && tid == 0) clk[2] = clock64();
 
                 // ---- 1: the runs of group g, record by record (raft.rs:1663-1743)
                 uint32_t p = s_run[gl];
@@ -380,7 +264,7 @@ __global__ void __launch_bounds__(kFTile *kFGroups + 64, 1) step_tile_compact_ke
                                 }
                             }
                         }
-                        if (general) res = tile_general_apply(c, rec, ext_hint, ext_snapshot, gl, hint, t, local);
+                        if (general) res = tile_general_apply<2>(c, rec, nullptr, ext_hint, ext_snapshot, gl, hint, t, local);
                         if (a.results) a.results[ua + p] = static_cast<uint8_t>(res);
                         p += step;
                     }
@@ -447,74 +331,26 @@ __global__ void __launch_bounds__(kFTile *kFGroups + 64, 1) step_tile_compact_ke
                                          : (RAFTGPU_META_IN(t.meta[gt]) | RAFTGPU_META_OUT(t.meta[gt]) | RAFTGPU_META_LEARN(t.meta[gt]));
                             general = !(fast_ok && tile_fast_apply<kSimple5>(c, t, gt, g0 + gt, slot, rec.index, rec.commit, is_local,
                                                                              is_reject, ext_hint, hint, present_mask, local, res));
-                            if (general) res = tile_general_apply(c, rec, ext_hint, ext_snapshot, gt, hint, t, local);
+                            if (general) res = tile_general_apply<2>(c, rec, nullptr, ext_hint, ext_snapshot, gt, hint, t, local);
                         }
                     }
                     if (a.results) a.results[ua + k] = static_cast<uint8_t>(res);
                 }
                 named_bar_sync(bar_id, kFTile);
                 if (a.dup_count && tid < kFTile / 4) s_touch[tid] = 0;  // clean for this consumer group's next tile
-                if (a.dbg && tid == 0) t2 = clock64();
+                if (a.dbg && tid == 0) clk[2] = clock64();
             }
             __syncwarp();
-            if (a.dbg && tid == 0) t3 = clock64();
+            if (a.dbg && tid == 0) clk[3] = clock64();
 
-            // ---- 2: Raft::maybe_commit for this thread's group (raft.rs:893-904)
-            {
-                bool advanced = false;
-                if (active) {
-                    const uint32_t meta = t.meta[gl];
-                    uint64_t v[kSlots];
-                    uint32_t r = 0;
-#pragma unroll
-                    for (int s2 = 0; s2 < kSlots; s2++) {
-                        v[s2] = 0;
-                        if ((hint >> s2) & 1u) {
-                            v[s2] = t.matched[r * R64 + gl];
-                            r++;
-                        }
-                    }
-                    uint64_t mci;
-                    bool use_gc;
-                    eval_mci<kSimple5>(c, g, meta, v, hint, mci, use_gc);
-                    advanced = mci > t.committed[gl] && mci >= t.ts[gl] && mci <= t.li[gl];  // raft_log.rs:488
-                    if (advanced) {
-                        t.committed[gl] = mci;  // (the store warp copies the row to commit_out too)
-                        if (meta & RAFTGPU_META_HAS_SELF) {  // raft.rs:896-900
-                            const uint32_t self = RAFTGPU_META_SELF(meta);
-                            uint64_t *pc = ((hint >> self) & 1u)
-                                               ? &t.pc[__popc(hint & ((1u << self) - 1u)) * R64 + gl]
-                                               : &c.peer_committed[static_cast<size_t>(self) * c.cap + g];
-                            if (mci > *pc) *pc = mci;
-                        }
-                    }
-                }
-                uint32_t lc[2] = {0, 0};
-                publish_tile(a.adv_bitmap, static_cast<uint64_t>(g0) + gl, lane, active, advanced, lc);
-                local[5] += lc[0];
-                local[6] += lc[1];
-            }
-
-            // ---- 3: hand the stage to the store warp
-            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-            named_bar_sync(bar_id, kFTile);
-            if (tid == 0) mbar_arrive(&done_bar[st]);
-            if (a.dbg && tid == 0) {
-                t4 = clock64();
-                atomicAdd(&a.dbg[0], static_cast<unsigned long long>(t1 - t0));  // waiting for the TMA loads
-                atomicAdd(&a.dbg[1], static_cast<unsigned long long>(t2 - t1));  // 0: run index
-                atomicAdd(&a.dbg[2], static_cast<unsigned long long>(t3 - t2));  // 1: records
-                atomicAdd(&a.dbg[3], static_cast<unsigned long long>(t4 - t3));  // 2 + 3: recompute, fence, barrier
-                atomicAdd(&a.dbg[4], 1ull);
-            }
+            // ---- 2: Raft::maybe_commit for this thread's group, 3: hand the stage to the store warp
+            tile_commit<kSimple5>(c, t, gl, g, ng, hint, lane, a.adv_bitmap, local);
+            tile_handoff(&bar.done[st], bar_id, tid);
+            // dbg: waiting for the TMA loads, 0: run index, 1: records, 2 + 3: recompute, fence, barrier
+            tile_debug(a.dbg, tid, clk);
         }
     }
-    const int which[7] = {kCntRecords, kCntUpdates, kCntRejects, kCntDecrements, kCntNoProgress, kCntRecomputes, kCntAdvanced};
-    block_flush_counts<7>(local, which, a.counters, nullptr);
-    if (a.step_advanced) {
-        const uint32_t w = __reduce_add_sync(0xffffffffu, local[6]);
-        if (lane == 0 && w) atomicAdd(a.step_advanced, w);
-    }
+    tile_flush(local, a);
 }
 
 // Tile index of a tileable compact stream, on the device (the zero-copy step has no host pass
